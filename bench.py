@@ -20,6 +20,11 @@ of the reference env would call): per step the caller's 16-bit words cross PCIe 
 place); the rank's envs are stepped as two shards (PipelinedChessEnv), one in flight while the host handles the other.
 `e2e.full_*` are the same loop carrying what step() returns to a learner: + the observation (32 B of bit-planes per env)
 and + the 528-byte legal-action bit mask per env.
+
+--dump-outputs DIR writes what the timed call (step_sampled) returned for its last step as float32 .npy files, so that two
+builds can be compared output for output: reward.npy, done.npy, flags.npy [N] (a seeded sample of DUMP_MAX_ENVS envs when
+N is larger) and observation.npy [DUMP_OBS_ENVS, 64], the board each env of a seeded sample was left with.  The envs,
+seeds and step counts depend only on the arguments, so the same arguments give the same inputs on every run.
 """
 import argparse
 import json
@@ -31,6 +36,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True   # the benchmark writes nothing into the tree, which may be read-only
 
 ENVS_PER_GPU = 524288
 METRIC = "env_steps_per_sec"
@@ -39,6 +45,8 @@ WORKLOAD = ("random self-play, opponent=none, auto-reset, on-device Philox actio
             "(BASELINE.json configs[3]: 4M envs over 8xB200, per-GPU shard)")
 CPU_SAMPLE_ENVS = 65536     # the CPU arm's bounded sample of the same workload
 PUBLISHED = {"steps_per_sec": 3205, "source": "gym_chess/test/v2/test_benchmark.py:46-50 (1851 steps in 0.5776 s, 1 thread, unspecified CPU)"}
+DUMP_MAX_ENVS = 1 << 20     # --dump-outputs: reward / done / flags of at most this many envs (12 MB of float32)
+DUMP_OBS_ENVS = 16384       # ... and the observation of this many (4 MB)
 
 
 def peaks():
@@ -52,6 +60,23 @@ def peaks():
 def median(xs):
     s = sorted(xs)
     return s[len(s) // 2]
+
+
+def dump_outputs(out_dir, env):
+    """--dump-outputs: reward / done / flags of the last step of the timed step_sampled call (the env's output buffers hold
+    them until it is stepped again) and the board observation that step left behind, as float32 out_dir/<name>.npy"""
+    import numpy as np
+
+    N = env.num_envs
+
+    def sample(k, seed):
+        return np.arange(N) if N <= k else np.sort(np.random.RandomState(seed).choice(N, k, replace=False))
+
+    idx = sample(DUMP_MAX_ENVS, 1)
+    arrays = {name: t.cpu().numpy()[idx] for name, t in (("reward", env.reward), ("done", env.done), ("flags", env.flags))}
+    arrays["observation"] = env.observe().reshape(N, 64).cpu().numpy()[sample(DUMP_OBS_ENVS, 2)]
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float32))
 
 
 class ClockSampler:
@@ -154,7 +179,10 @@ def main():
     ap.add_argument("--envs-per-gpu", type=int, default=ENVS_PER_GPU)
     ap.add_argument("--burn-in", type=int, default=600, help="untimed steps after the phases have been spread")
     ap.add_argument("--no-extras", action="store_true", help="skip the movegen / small-config / cpu_baseline legs")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step to DIR/<name>.npy (rank 0)")
     args = ap.parse_args()
+    if args.dump_outputs:
+        os.makedirs(args.dump_outputs, exist_ok=True)
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -227,6 +255,9 @@ def main():
     launches = (L.gcb_launch_count() - launches0) // R
     ms = median(rep_ms)
     st = env.stats()
+    assert st["steps"] == N * K * R, (st["steps"], N, K, R)   # every repeat stepped every env exactly K times
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, env)
     value = world * N * K / (ms * 1e-3)
 
     # ---- final NCCL reduce of the episode statistics (the only collective of the job)
