@@ -108,6 +108,7 @@ SIGNATURES = {
     "gcb_env_destroy": (i32, [vp]),
     "gcb_env_reset": (i32, [vp, vp, vp]),
     "gcb_env_import": (i32, [vp, vp, vp, vp, vp, vp, vp]),
+    "gcb_env_clone": (i32, [vp, vp, vp, vp]),
     "gcb_env_step": (i32, [vp, vp, vp, vp, vp, vp]),
     "gcb_env_step_index": (i32, [vp, vp, vp, vp, vp, vp]),
     "gcb_env_bot_ply": (i32, [vp, vp, vp, vp, vp, vp]),

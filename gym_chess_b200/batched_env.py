@@ -66,6 +66,8 @@ class BatchedChessEnv:
         self.device = torch.device("cuda", device) if not isinstance(device, torch.device) else device
         self.auto_reset, self.seed, self.env_id_offset = bool(auto_reset), int(seed), int(env_id_offset)
         self.legal_stride = int(legal_stride)
+        self.history_cap = int(history_cap) or 512  # (resolved like gcb_env_create does)
+        self.moves_max = 149 if moves_max < 0 else int(moves_max)
         cfg = EnvConfig()
         cfg.num_envs, cfg.env_id_offset, cfg.seed = self.num_envs, self.env_id_offset, self.seed
         cfg.opponent, cfg.agent_black, cfg.auto_reset = _OPPONENTS[opponent], int(player_color == BLACK), int(auto_reset)
@@ -120,6 +122,39 @@ class BatchedChessEnv:
             check(_lib.lib().gcb_env_import(self._h, C.c_void_p(b.data_ptr()), C.c_void_p(p.data_ptr()), C.c_void_p(r.data_ptr()),
                                             C.c_void_p(mc.data_ptr()) if mc is not None else None,
                                             C.c_void_p(m.data_ptr()) if m is not None else None, _stream_ptr()))
+
+    def clone_from(self, source, index):
+        """Per-env clone (branching a game mid-episode: search rollouts, lookahead, duplicating games): env j becomes env
+        index[j] of `source` (a BatchedChessEnv, possibly self) for every j with 0 <= index[j] < source.num_envs; rows with
+        index[j] < 0 are left untouched, repeated indices fan one source env out.  index int [num_envs] (tensor or array).
+        Unlike set_state the clone continues the source's episode: board, counters, done, an owed bot ply and the repetition
+        window (a clone scores a 3-fold repetition exactly as its source would).  Env j keeps its global id, seed, templates and
+        statistics; its episode counter advances by one, so its random draws differ from the source's and from an earlier clone
+        into the same row.  Both envs must agree in history_cap, piece slots, opponent, player_color and moves_max.  With
+        source = self, no selected row may also be the source of a selected row."""
+        if not isinstance(source, BatchedChessEnv):
+            raise ValueError("clone_from: source must be a BatchedChessEnv")
+        if source.device != self.device:
+            raise ValueError("clone_from: source lives on %s, this env on %s" % (source.device, self.device))
+        for name, mine, theirs in (("history_cap", self.history_cap, source.history_cap),
+                                   ("piece slots", self._n_slots(), source._n_slots()), ("opponent", self.opponent, source.opponent),
+                                   ("player_color", self.player_color, source.player_color),
+                                   ("moves_max", self.moves_max, source.moves_max)):
+            if mine != theirs:
+                raise ValueError("clone_from: %s differs (%r here, %r in the source)" % (name, mine, theirs))
+        idx = torch.as_tensor(index, device=self.device)
+        if tuple(idx.shape) != (self.num_envs,):
+            raise ValueError("clone_from: index must have shape [%d], got %s" % (self.num_envs, list(idx.shape)))
+        if idx.dtype.is_floating_point or idx.dtype == torch.bool:
+            raise ValueError("clone_from: index must be an integer tensor")
+        idx = idx.to(torch.int32).contiguous()
+        with torch.cuda.device(self.device):
+            check(_lib.lib().gcb_env_clone(self._h, source._h, C.c_void_p(idx.data_ptr()), _stream_ptr()))
+
+    def _n_slots(self):
+        n = C.c_int32()
+        check(_lib.lib().gcb_env_piece_slots(self._h, None, C.byref(n)))
+        return n.value
 
     def _outs(self):
         return C.c_void_p(self.reward.data_ptr()), C.c_void_p(self.done.data_ptr()), C.c_void_p(self.flags.data_ptr())

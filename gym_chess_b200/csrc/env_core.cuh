@@ -50,7 +50,10 @@ __device__ unsigned long long g_violations = 0ULL;
     do {                    \
     } while (0)
 #endif
-enum { CHK_STAT_ROW = 0, CHK_ENV_INDEX = 1, CHK_SLOT_INDEX = 2, CHK_REP_INDEX = 3, CHK_IO_INDEX = 4, CHK_LIST_INDEX = 5 };
+// CHK_CLONE_INDEX: a clone index >= the source's env count (the row is left alone in both builds); CHK_CLONE_ALIAS: a clone
+// destination row that is also the source row of some destination of the same call
+enum { CHK_STAT_ROW = 0, CHK_ENV_INDEX = 1, CHK_SLOT_INDEX = 2, CHK_REP_INDEX = 3, CHK_IO_INDEX = 4, CHK_LIST_INDEX = 5,
+       CHK_CLONE_INDEX = 6, CHK_CLONE_ALIAS = 7 };
 
 // The resident state is touched once per step: stream it past L1 (ld.global.cs / st.global.cs, evict-first) so that
 // the geometry tables the generation hammers stay L1-resident.
@@ -770,6 +773,53 @@ GCB_HD void env_import_one(const EnvView& v, int e, const int8_t* board, int pla
     bool rep;
     ply_and_movegen(v, e, s, 0, false, &rep, st, scratch, resident_slots(v, e), GeomGlobal());
     env_store(v, e, s, ep + 1u);
+}
+
+// Clone (gcb_env_clone): env d of `dst` becomes env i of `src` mid-episode -- board, key, meta (done, counters, hist_len,
+// bot_pending), count bytes, piece slots and the live entries of the repetition window.  The destination keeps its global id,
+// seed, templates and statistics rows; its episode counter advances by one (a re-clone into the same row draws new words) and
+// its window moves to a new generation G = its old generation + 1, under which every entry it held before is dead.  The three
+// parts below are what one warp of k_env_clone splits among its lanes; env_clone_one runs them in sequence.
+//
+// The per-env words of the clone.  Returns G; *src_gen / *src_hist receive the source's generation and window length.
+GCB_HD u32 env_clone_words(const EnvView& dst, int d, const EnvView& src, int i, u32* src_gen, int* src_hist) {
+    EnvRegs s;
+    u32 ep;
+    env_load(src, i, s, ep);
+    *src_gen = s.gen, *src_hist = s.hist_len;
+    GCB_CHK((unsigned)d < (unsigned)dst.N, CHK_ENV_INDEX);
+    s.gen = GCB_LDS(&dst.gen[d]) + 1u;
+    env_store(dst, d, s, GCB_LDS(&dst.episode[d]) + 1u);
+    return s.gen;
+}
+// piece slot r of the clone
+GCB_HD void env_clone_slot(const EnvView& dst, int d, const EnvView& src, int i, int r) {
+    const TgtSink from(resident_slots(src, i), nullptr);
+    TgtSink to(resident_slots(dst, d), nullptr);
+    to.st(r, from.get(r));
+}
+// one repetition-table entry of the source, retagged in place for the destination's generation G: true if it is live (and
+// must be written to the SAME slot of the destination's table -- live entries keep their slots and hence their probe chains;
+// nothing is ever deleted within a generation, and the overflow replacement of rep_lookup_insert keeps chains intact)
+GCB_HD bool rep_clone_entry(ulonglong2& en, u32 src_gen, u32 G) {
+    const u64 c = en.y & 3ULL;
+    if ((en.y >> 2) != (u64)src_gen || c == 0) return false;
+    en.y = ((u64)G << 2) | c;
+    return true;
+}
+GCB_HD void env_clone_one(const EnvView& dst, int d, const EnvView& src, int i) {
+    u32 sgen;
+    int hist;
+    const u32 G = env_clone_words(dst, d, src, i, &sgen, &hist);
+    for (int r = 0; r < dst.slots; r++) env_clone_slot(dst, d, src, i, r);
+    if (hist == 0) return;  // an empty window: every source entry is dead, nothing to read
+    const size_t H2 = (size_t)src.hist_mask + 1;
+    const ulonglong2* from = src.rep + (size_t)i * H2;
+    ulonglong2* to = dst.rep + (size_t)d * H2;
+    for (size_t k = 0; k < H2; k++) {
+        ulonglong2 en = GCB_LDS(&from[k]);
+        if (rep_clone_entry(en, sgen, G)) GCB_STS(&to[k], en);
+    }
 }
 
 // initial state of one template board (ChessEnvV2.reset up to the first movegen, chess_v2.py:188-206)

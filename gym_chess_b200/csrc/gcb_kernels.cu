@@ -456,6 +456,58 @@ __global__ void __launch_bounds__(GCB_BLOCK) k_env_import(EnvView v, const int8_
     env_import_one(v, e, m, players[e], rights, move_count ? move_count[e] : 0, st, &s_counts[threadIdx.x]);
 }
 
+// gcb_env_clone, one warp per destination row d (env_clone_* of env_core.cuh split among the lanes): lane 0 copies the ~70 B
+// of per-env words and broadcasts the source's generation and window length, lane r copies piece slot r (slot-major: the
+// lanes of neighbouring warps fill the same 32-byte sectors), and when the source's window is non-empty all 32 lanes sweep
+// its 2H-entry table, 16 B per lane and load, eight loads in flight per lane before any store, writing only the live entries
+// (retagged to the destination's new generation).  is_src (CHECKED build, in-object clones only): 1 where a row is the source
+// of some selected destination (k_env_clone_mark).
+#define GCB_CLONE_BATCH 8
+__global__ void __launch_bounds__(GCB_BLOCK) k_env_clone(EnvView dst, EnvView src, const int32_t* __restrict__ index,
+                                                         const uint8_t* __restrict__ is_src) {
+    const int d = (int)((blockIdx.x * (unsigned)blockDim.x + threadIdx.x) >> 5), lane = threadIdx.x & 31;
+    if (d >= dst.N) return;
+    const int i = __ldg(index + d);
+    if (i < 0) return;
+    GCB_CHK(i < src.N, CHK_CLONE_INDEX);
+    if (i >= src.N) return;
+    (void)is_src;
+#if defined(GCB_CHECKED)
+    if (is_src) GCB_CHK(!is_src[d], CHK_CLONE_ALIAS);
+#endif
+    u32 sgen = 0, G = 0;
+    int hist = 0;
+    if (lane == 0) G = env_clone_words(dst, d, src, i, &sgen, &hist);
+    for (int r = lane; r < dst.slots; r += 32) env_clone_slot(dst, d, src, i, r);
+    sgen = __shfl_sync(0xffffffffu, sgen, 0), G = __shfl_sync(0xffffffffu, G, 0), hist = __shfl_sync(0xffffffffu, hist, 0);
+    if (hist == 0) return;
+    const unsigned H2 = (unsigned)src.hist_mask + 1u;  // 2H >= 16 entries, a multiple of 16
+    const ulonglong2* from = src.rep + (size_t)i * H2;
+    ulonglong2* to = dst.rep + (size_t)d * H2;
+#pragma unroll 1
+    for (unsigned k0 = lane; k0 < H2; k0 += 32u * GCB_CLONE_BATCH) {
+        ulonglong2 en[GCB_CLONE_BATCH];
+#pragma unroll
+        for (int b = 0; b < GCB_CLONE_BATCH; b++) {
+            const unsigned k = k0 + 32u * b;
+            en[b] = k < H2 ? __ldcs(&from[k]) : make_ulonglong2(0ULL, 0ULL);
+        }
+#pragma unroll
+        for (int b = 0; b < GCB_CLONE_BATCH; b++) {
+            const unsigned k = k0 + 32u * b;
+            if (k < H2 && rep_clone_entry(en[b], sgen, G)) __stcs(&to[k], en[b]);
+        }
+    }
+}
+
+// CHECKED build, in-object clone: mark the source row of every selected destination (the aliasing check of k_env_clone)
+__global__ void k_env_clone_mark(int n, int src_n, const int32_t* __restrict__ index, uint8_t* __restrict__ is_src) {
+    const int d = blockIdx.x * blockDim.x + threadIdx.x;
+    if (d >= n) return;
+    const int i = index[d];
+    if (i >= 0 && i < src_n) is_src[i] = 1;
+}
+
 __global__ void k_init_zobrist(u64* tab) {
     int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i < GCB_ZOB_ENTRIES) fill_zobrist_entry(tab, i);
@@ -1244,6 +1296,31 @@ extern "C" int gcb_env_import(gcb_env* env, const int8_t* d_boards, const int8_t
     env->tick++;
     LAUNCHED();
     return refresh_mask_output(env, (cudaStream_t)stream);
+}
+
+extern "C" int gcb_env_clone(gcb_env* dst, const gcb_env* src, const int32_t* d_src_index, void* stream) {
+    ENV_CHECK(dst);
+    if (!src || !d_src_index) return fail(GCB_E_ARG, "gcb_env_clone", "null pointer");
+    const gcb_env_config &a = dst->cfg, &b = src->cfg;
+    if (a.device != b.device) return fail(GCB_E_ARG, "gcb_env_clone", "source and destination live on different devices");
+    if (a.piece_slots != b.piece_slots || a.history_cap != b.history_cap || a.opponent != b.opponent ||
+        a.agent_black != b.agent_black || a.moves_max != b.moves_max)
+        return fail(GCB_E_ARG, "gcb_env_clone", "source and destination differ in piece_slots, history_cap, opponent, agent colour or moves_max");
+    const cudaStream_t s = (cudaStream_t)stream;
+    uint8_t* is_src = nullptr;
+#if defined(GCB_CHECKED)
+    if (src == dst) {  // the aliasing check: which rows are sources of this call
+        CU(cudaMallocAsync((void**)&is_src, (size_t)dst->v.N, s));
+        CU(cudaMemsetAsync(is_src, 0, (size_t)dst->v.N, s));
+        k_env_clone_mark<<<grid_for(dst->v.N), GCB_BLOCK, 0, s>>>(dst->v.N, src->v.N, d_src_index, is_src);
+        LAUNCHED();
+    }
+#endif
+    const int warps_per_block = GCB_BLOCK / 32;
+    k_env_clone<<<(dst->v.N + warps_per_block - 1) / warps_per_block, GCB_BLOCK, 0, s>>>(dst->v, src->v, d_src_index, is_src);
+    LAUNCHED();
+    if (is_src) CU(cudaFreeAsync(is_src, s));
+    return refresh_mask_output(dst, s);
 }
 
 // ---- checkpoint / resume: the resident state is plain arrays; a snapshot is their concatenation in one device buffer

@@ -153,6 +153,28 @@ int gcb_env_reset(gcb_env *env, const uint8_t *d_mask, void *stream);
 int gcb_env_import(gcb_env *env, const int8_t *d_boards, const int8_t *d_players, const uint8_t *d_rights4,
                    const int32_t *d_move_count, const uint8_t *d_mask, void *stream);
 
+/* Per-env clone: branch games mid-episode (search rollouts, lookahead, duplicating games of a batch).  d_src_index int32[N of
+ * dst] (device): for every destination row j of `dst` with 0 <= d_src_index[j] < src's N, env j of `dst` becomes env
+ * i = d_src_index[j] of `src`.  Rows with a negative index are left untouched (this takes the place of a mask; fan-out is
+ * repeated indices).  Unlike gcb_env_import, the clone continues the source's EPISODE, repetition window included:
+ *   copied from the source: board planes, Zobrist key, meta (side to move, rights, check flags, done, castle bits, n_legal,
+ *     move_count, step_in_episode, hist_len, bot_pending), count bytes, all piece slots, and the live entries of the
+ *     repetition table;
+ *   kept from the destination: global env id and seed (the Philox draws of a clone differ from its source's), templates
+ *     (used by a later auto-reset), statistics rows (a clone is not a step: no counter moves);
+ *   episode counter: the destination's own + 1, like gcb_env_import (re-cloning a root into the same row does not replay the
+ *     same random words);
+ *   repetition table: new generation G = the destination's generation + 1; every live source entry is written to the SAME
+ *     slot of the destination's table, retagged to G, and nothing else is written (the destination's older entries are dead
+ *     under G; a source with an empty window needs no table read).
+ * src and dst must live on the same device and agree in the resolved piece_slots, history_cap, opponent, agent_black and
+ * moves_max (GCB_E_ARG otherwise); num_envs, seed, env_id_offset, auto_reset and templates may differ.  src == dst is
+ * allowed, but no selected destination row may also be the source row of a selected destination (the result is then
+ * unspecified).  An index >= src's N leaves its row untouched; the CHECKED build additionally records it (and the aliasing
+ * case) through gcb_debug_violations.  Enqueued on `stream`: ordering against work on `src` on other streams is the
+ * caller's.  A mask output registered on dst (gcb_env_step_mask_output) is current afterwards. */
+int gcb_env_clone(gcb_env *dst, const gcb_env *src, const int32_t *d_src_index, void *stream);
+
 /* ChessEnvV2.step(action), chess_v2.py:219-294, for all N envs.  Outputs (device, any may be NULL):
  * d_reward int32[N] (the two float 0.0 literals are 0), d_done uint8[N], d_flags uint8[N] (GCB_F_*). */
 int gcb_env_step(gcb_env *env, const int32_t *d_actions, int32_t *d_reward, uint8_t *d_done, uint8_t *d_flags,
