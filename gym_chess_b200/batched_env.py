@@ -23,7 +23,7 @@ STAT_NAMES = ("steps", "plies", "episodes", "mates", "repetitions", "caps", "wed
               "legal_sum", "in_check", "hist_overflow", "slot_overflow", "hist_scanned", "hist_window")
 INFO_NAMES = ("current_player", "white_king_castle_is_possible", "white_queen_castle_is_possible",
               "black_king_castle_is_possible", "black_queen_castle_is_possible", "white_king_is_checked",
-              "black_king_is_checked", "done", "move_count", "n_legal", "episode", "step_in_episode", "hist_len", "castles")
+              "black_king_is_checked", "done", "move_count", "n_legal", "episode", "step_in_episode", "hist_len", "castles", "bot_pending")
 
 
 class _DevArray:
@@ -54,7 +54,8 @@ class BatchedChessEnv:
         opponent      "random" (the bot replies inside step, chess_v2.py:277-288; drawn on the device), "none" (self-play)
                       or "external" (a callable opponent, chess_v2.py:171-179: step() stops with F_BOT_PENDING where the
                       bot would move and the caller supplies its ply with bot_ply())
-        player_color  "WHITE" | "BLACK" (BLACK needs opponent="random", like the reference: Q23)
+        player_color  "WHITE" | "BLACK" (BLACK needs a bot to open for White, opponent "random" or "external", like the
+                      reference: Q23)
         initial_boards  None (DEFAULT_BOARD) or int8 [T,8,8] / [8,8]; env with global id g starts from board g % T
         env_id_offset   global id of local env 0 -- shards of one job use disjoint id ranges so that the
                         Philox draws (counter = global env id, episode, step) do not depend on the sharding
@@ -160,15 +161,22 @@ class BatchedChessEnv:
         return C.c_void_p(self.reward.data_ptr()), C.c_void_p(self.done.data_ptr()), C.c_void_p(self.flags.data_ptr())
 
     def step(self, actions):
-        """actions: int32 [N] cuda tensor.  -> (reward int32[N], done uint8[N], flags uint8[N]) (reused buffers)."""
+        """actions: int32 [N] cuda tensor.  -> (reward int32[N], done uint8[N], flags uint8[N]) (reused buffers).
+        opponent="external": F_BOT_PENDING marks the envs that owe the bot a ply when the call returns (see bot_ply)."""
         a = torch.as_tensor(actions, device=self.device).to(torch.int32).contiguous()
         with torch.cuda.device(self.device):
             check(_lib.lib().gcb_env_step(self._h, C.c_void_p(a.data_ptr()), *self._outs(), _stream_ptr()))
         return self.reward, self.done, self.flags
 
     def bot_ply(self, bot_actions):
-        """opponent="external": the bot's ply of every env that owes one (F_BOT_PENDING / after a BLACK-agent reset), applied
-        like the reference applies opponent_policy(env).  -> (reward to ADD, done, flags), valid for the envs that owed a ply."""
+        """opponent="external": the bot's ply of every env that owes one, applied like the reference applies
+        opponent_policy(env) (no membership test).  An env owes a ply exactly when the last step / bot_ply output of its row
+        carried F_BOT_PENDING (and after reset() with player_color BLACK; info column bot_pending): the reply to the agent's
+        ply, or White's opening of a new BLACK-agent episode.  -> (reward, done, flags), written only for the envs that owed a ply:
+        for a reply the reward is to be ADDED to that of the agent's half; the opening reports 0, not done, no flags (the
+        reference's reset discards it).  flags carry F_BOT_PENDING again when an auto-reset started a BLACK-agent episode.
+        Envs that owe nothing are left alone, their output rows untouched.  A step() of an env that owes a ply is refused:
+        reward -10, F_INVALID | F_BOT_PENDING, state unchanged."""
         a = torch.as_tensor(bot_actions, device=self.device).to(torch.int32).contiguous()
         with torch.cuda.device(self.device):
             check(_lib.lib().gcb_env_bot_ply(self._h, C.c_void_p(a.data_ptr()), *self._outs(), _stream_ptr()))
@@ -231,8 +239,9 @@ class BatchedChessEnv:
     def _host_async(self, fn, inp, reward, done, flags, stream):
         check(fn(self._h, _host_ptr(inp), _host_ptr(reward), _host_ptr(done), _host_ptr(flags), _stream_ptr(stream)))
 
-    # packed 16-bit records (2 bytes in, 2 bytes out per env): uint16 actions / random words, uint16 results; buffers are
-    # cuda tensors or page-locked host tensors / arrays; asynchronous like the calls above
+    # packed 16-bit records (2 bytes in, 2 bytes out per env): uint16 actions / random words, uint16 results (bits 0-7 reward
+    # as int8, bits 8-14 the flags F_INVALID .. F_BOT_PENDING, bit 15 done); buffers are cuda tensors or page-locked host
+    # tensors / arrays; asynchronous like the calls above
     def step_packed(self, actions16, result16, stream=None):
         check(_lib.lib().gcb_env_step_packed(self._h, _host_ptr(actions16), _host_ptr(result16), _stream_ptr(stream)))
 
@@ -243,7 +252,7 @@ class BatchedChessEnv:
     def unpack_result(result16):
         """uint16 records -> (reward int32, done uint8, flags uint8); numpy array or torch tensor (viewed as int16/int32)"""
         r = np.asarray(result16).view(np.uint16) if not isinstance(result16, torch.Tensor) else result16.cpu().numpy().view(np.uint16)
-        return (r & 0xFF).astype(np.uint8).view(np.int8).astype(np.int32), (r >> 15).astype(np.uint8), ((r >> 8) & 63).astype(np.uint8)
+        return (r & 0xFF).astype(np.uint8).view(np.int8).astype(np.int32), (r >> 15).astype(np.uint8), ((r >> 8) & 127).astype(np.uint8)
 
     def wait(self, stream=None):
         """block until the steps enqueued on `stream` (default: the current torch stream) have finished"""

@@ -513,7 +513,7 @@ struct StepIO {
     int nsteps;          // MODE_SAMPLED: consecutive steps run by ONE launch (envs are independent: no grid-wide sync needed)
     // packed 16-bit records (host-buffer steps are bound by the bytes that cross PCIe): in16 != 0 -> `in` holds uint16
     // actions / uint16 random words (a word w draws like the 32-bit word w << 16); packed != NULL -> one uint16 result
-    // per env: bits 0-7 reward (int8; a reward is always within [-120, 100]), bits 8-13 flags, bit 15 done
+    // per env: bits 0-7 reward (int8; a reward is always within [-120, 100]), bits 8-14 flags, bit 15 done
     uint16_t* packed = nullptr;
     int in16 = 0;
     // learner-facing output of the step itself: possible_actions of the state the step leaves behind as the 65-word bit
@@ -532,7 +532,7 @@ GCB_HD u32 step_input(const StepIO& io, int e) {
     return 0u;
 }
 GCB_HD uint16_t pack_result(int reward, bool done, u32 flags) {
-    return (uint16_t)((u32)(reward & 0xFF) | ((flags & 63u) << 8) | (done ? 0x8000u : 0u));
+    return (uint16_t)((u32)(reward & 0xFF) | ((flags & 127u) << 8) | (done ? 0x8000u : 0u));
 }
 
 // resident state of env e <-> registers
@@ -589,6 +589,8 @@ GCB_HD void env_step_regs(const EnvView& v, const StepIO& io, int e, EnvRegs& s,
         s.pending = 0;
         action = bot_action = (int)input;
         agent_ply = true;
+        // the opening after a reset is owed at step 0 and only there: a step refused because a ply is owed does not advance
+        // step_in_episode, a played step does before it can leave a reply owed (a state import starts at 0 but owes nothing)
         phase = (s.step == 0 && v_agent_black) ? PH_RESETBOT : PH_BOT;
     } else {
         bool valid = false;
@@ -608,9 +610,12 @@ GCB_HD void env_step_regs(const EnvView& v, const StepIO& io, int e, EnvRegs& s,
                 }
             }
         }
-        if (!SELFPLAY && s.pending) valid = false;  // a bot ply is owed first: the agent's action is refused
+        // a bot ply is owed first: the agent's action is refused and step_in_episode does not advance; the statistics count
+        // the call as a step and as an invalid one
+        const bool refused = !SELFPLAY && s.pending;
+        if (refused) valid = false;
         st.f += SF_STEPS + (stm_checked(s) ? SF_INCHECK : 0u), st.legal += n0;
-        s.step++;
+        if (!refused) s.step++;
         if (!valid) {  // chess_v2.py:240-242, before the done test (Q16)
             R = -10, d_out = s.done, fl |= EF_INVALID, st.f += SF_INVALID;
             phase = PH_FINAL;
@@ -651,8 +656,10 @@ GCB_HD void env_step_regs(const EnvView& v, const StepIO& io, int e, EnvRegs& s,
             } else {
                 if (agent_ply) d_out = s.done;
                 terminal = !owe_bot && (d_out || s.n_legal == 0);
-                if (owe_bot) fl |= EF_BOT_PENDING;
-                else if (!d_out && s.n_legal == 0) fl |= EF_WEDGED;
+                if (!owe_bot && !d_out && s.n_legal == 0) fl |= EF_WEDGED;
+                // F_BOT_PENDING = the env owes the bot a ply when the call returns: the reply to this step's ply, a ply still
+                // owed (a refused step) or the opening of the BLACK-agent episode an auto-reset starts
+                if (v_ext && ((v.auto_reset && terminal) ? v_agent_black : s.pending)) fl |= EF_BOT_PENDING;
                 if (n0 == 0 || was_done || owe_bot || (fl & EF_INVALID)) {
                 } else if (capped) st.f += SF_CAPS;
                 else if (d_out) {
@@ -666,7 +673,8 @@ GCB_HD void env_step_regs(const EnvView& v, const StepIO& io, int e, EnvRegs& s,
                 if (io.reward) io.reward[e] = R;
                 if (io.done) io.done[e] = d_out ? 1 : 0;
                 if (io.flags) io.flags[e] = (uint8_t)fl;
-                if (io.packed) io.packed[e] = pack_result(R, d_out, fl);
+                // (self-play sets no flag above F_RESET; saying so keeps the self-play kernels' packing as it was)
+                if (io.packed) io.packed[e] = pack_result(R, d_out, SELFPLAY ? fl & 63u : fl);
                 if (io.act_out) io.act_out[e] = action;
             }
             if ((MODE == MODE_RESET) || (v.auto_reset && terminal)) {
@@ -739,6 +747,15 @@ GCB_HD void env_step_regs(const EnvView& v, const StepIO& io, int e, EnvRegs& s,
         } else {                // PH_RESETBOT
             s.move_count += 1;  // chess_v2.py:214
             s.done = 0;
+            if (MODE == MODE_BOTPLY) {
+                // the caller's opening ply: the reference's reset discards its reward and clears done, and nothing is owed after it
+                GCB_CHK((unsigned)e < (unsigned)v.N, CHK_IO_INDEX);
+                if (io.reward) io.reward[e] = 0;
+                if (io.done) io.done[e] = 0;
+                if (io.flags) io.flags[e] = 0;
+                if (io.packed) io.packed[e] = pack_result(0, false, 0u);
+                if (io.act_out) io.act_out[e] = action;
+            }
             phase = PH_END;
         }
     }

@@ -177,7 +177,7 @@ class ChessEnvV2:
         if played and self.log and not (flags & F_REPETITION):
             self._log_ply(self.action_to_move(action))
         self._pull()
-        if flags & F_BOT_PENDING:  # chess_v2.py:277-288
+        if flags & F_BOT_PENDING and not flags & F_INVALID:  # chess_v2.py:277-288 (a refused step plays no ply: no reply)
             r2, done = self._bot_ply()
             reward += r2
         return self.state, reward, done, self.info

@@ -53,7 +53,9 @@ extern "C" {
                                 terminates here (stalemate is not a terminal state; with the random bot it raises
                                 TypeError).  Reported so that callers / auto-reset can act on it. */
 #define GCB_F_RESET 32u      /* the env was auto-reset after this step */
-#define GCB_F_BOT_PENDING 64u /* opponent 2 (external): the agent's ply is done, the bot's ply is owed (gcb_env_bot_ply) */
+#define GCB_F_BOT_PENDING 64u /* opponent 2 (external): the env owes the bot a ply when the call returns (gcb_env_bot_ply):
+                                 the reply to the agent's ply of this step, a ply still owed (the step was refused), or the
+                                 opening of the BLACK-agent episode an auto-reset started */
 
 const char *gcb_last_error(void);
 int gcb_version(void);
@@ -176,14 +178,22 @@ int gcb_env_import(gcb_env *env, const int8_t *d_boards, const int8_t *d_players
 int gcb_env_clone(gcb_env *dst, const gcb_env *src, const int32_t *d_src_index, void *stream);
 
 /* ChessEnvV2.step(action), chess_v2.py:219-294, for all N envs.  Outputs (device, any may be NULL):
- * d_reward int32[N] (the two float 0.0 literals are 0), d_done uint8[N], d_flags uint8[N] (GCB_F_*). */
+ * d_reward int32[N] (the two float 0.0 literals are 0), d_done uint8[N], d_flags uint8[N] (GCB_F_*).
+ * Opponent 2 (external): the step of an env that owes a bot ply is refused -- reward -10, done unchanged, GCB_F_INVALID |
+ * GCB_F_BOT_PENDING, and the env's state is left as it was (step_in_episode included; only an env whose bot has no legal
+ * move is reported GCB_F_WEDGED and auto-reset); the statistics count a step and an invalid action.  GCB_F_BOT_PENDING is
+ * set on every output of an env that owes a ply when the call returns. */
 int gcb_env_step(gcb_env *env, const int32_t *d_actions, int32_t *d_reward, uint8_t *d_done, uint8_t *d_flags,
                  void *stream);
-/* The bot's ply of an env created with opponent 2 (external), for every env that owes one (after a step that reported
- * GCB_F_BOT_PENDING, or after a reset with agent_black): d_bot_actions int32[N] is applied the way the reference applies
+/* The bot's ply of an env created with opponent 2 (external), for every env that owes one (after an output that reported
+ * GCB_F_BOT_PENDING, or after gcb_env_reset with agent_black): d_bot_actions int32[N] is applied the way the reference applies
  * opponent_policy(env) -- player_move without a membership test (chess_v2.py:277-288, 208-216).  Outputs like gcb_env_step,
- * written only for envs that owed a ply: d_reward = -(the bot's capture value) - 100 if the agent is mated (to be ADDED to
- * the reward of the agent's half), d_done, d_flags.  Envs that owe nothing are left alone. */
+ * written only for envs that owed a ply:
+ *   the reply to the agent's ply: d_reward = -(the bot's capture value) - 100 if the agent is mated (to be ADDED to the
+ *     reward of the agent's half), d_done, d_flags (GCB_F_BOT_PENDING when an auto-reset started a BLACK-agent episode);
+ *   White's opening of a BLACK-agent episode (owed from the reset until this call, however many steps were refused
+ *     meanwhile): reward 0, done 0, flags 0 -- the reference's reset discards the opening's reward and clears done.
+ * Envs that owe nothing are left alone: no state change, their output rows are not written. */
 int gcb_env_bot_ply(gcb_env *env, const int32_t *d_bot_actions, int32_t *d_reward, uint8_t *d_done, uint8_t *d_flags,
                     void *stream);
 /* same, but env i plays possible_actions[i][(u32[i] * n_legal[i]) >> 32] (RESIGN when it has no legal move): the uniform
@@ -223,7 +233,8 @@ int gcb_env_wait(gcb_env *env, void *stream);
  * memory fabric.  actions16 uint16[N] (an action code is < 4101); u16 uint16[N]: word w draws like the 32-bit word
  * w << 16 of gcb_env_step_index, i.e. possible_actions[(w * n_legal) >> 16]; result16 uint16[N]: bits 0-7 the reward as
  * int8 (a step's reward is always within [-120, 100]: -10, a capture <= 10, +-100 for a mate, minus the bot's capture),
- * bits 8-13 the GCB_F_* flags, bit 15 done.  Each pointer may be device memory or page-locked host memory (read / written
+ * bits 8-14 the GCB_F_* flags (GCB_F_INVALID .. GCB_F_BOT_PENDING: flag f sits at bit 8 + log2 f), bit 15 done.  An
+ * external-opponent env is stepped like with gcb_env_step, and bit 14 tells which envs owe gcb_env_bot_ply.  Each pointer may be device memory or page-locked host memory (read / written
  * in place through its device alias); results are valid after gcb_env_wait / a synchronisation of the stream. */
 int gcb_env_step_packed(gcb_env *env, const uint16_t *actions16, uint16_t *result16, void *stream);
 int gcb_env_step_index_packed(gcb_env *env, const uint16_t *u16, uint16_t *result16, void *stream);
@@ -231,7 +242,8 @@ int gcb_env_step_index_packed(gcb_env *env, const uint16_t *u16, uint16_t *resul
 /* observation / state export (device pointers, any may be NULL):
  *   d_boards int8[N][64]   -- `state["board"]`, the Box(-6,6,(8,8)) observation
  *   d_info   int32[N][16]  -- current_player(+1/-1), wk, wq, bk, bq, wchk, bchk, done, move_count, n_legal,
- *                             episode, step_in_episode, hist_len, castle bits (1 queen side | 2 king side), 0, 0 */
+ *                             episode, step_in_episode, hist_len, castle bits (1 queen side | 2 king side),
+ *                             bot_pending (opponent 2: a gcb_env_bot_ply is owed), 0 */
 int gcb_env_export(gcb_env *env, int8_t *d_boards, int32_t *d_info, void *stream);
 /* legal action mask uint8[N][4101] (possible_actions as a mask) */
 int gcb_env_legal_mask(gcb_env *env, uint8_t *d_mask, void *stream);

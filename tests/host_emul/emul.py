@@ -43,6 +43,8 @@ def lib():
         L.emul_env_export.argtypes = [vp, vp, vp, vp, C.c_int]
         L.emul_env_import.argtypes = [vp] * 6
         L.emul_env_stats.argtypes = [vp, vp]
+        L.emul_pack_result.argtypes = [C.c_int, C.c_int, C.c_uint32]
+        L.emul_pack_result.restype = C.c_uint16
         _lib = L
     return _lib
 

@@ -235,4 +235,7 @@ void emul_env_export(EmulEnv* E, int8_t* boards, int32_t* info, uint16_t* legal,
 
 void emul_env_stats(EmulEnv* E, uint64_t* out16) { memcpy(out16, E->v.stats, ST_COUNT * 8); }
 
+// the 16-bit result record of the packed step forms (gcb_env_step_packed)
+uint16_t emul_pack_result(int reward, int done, uint32_t flags) { return pack_result(reward, done != 0, flags); }
+
 }  // extern "C"
