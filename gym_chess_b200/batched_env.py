@@ -217,6 +217,54 @@ class BatchedChessEnv:
             self.step_sampled(max(1, period // groups))
             self.reset(ids % groups == g)
 
+    def sample_policy(self, logits, temperature=1.0, u32=None):
+        """Act from a learned policy: for every env, a legal action of the side to move drawn from `logits` (cuda float32 or
+        bfloat16 [N, >= 4101] on this env's device, last-dim stride 1; only the entries of legal actions are read).
+        -> (actions int32[N], logp float32[N]).  temperature T > 0 samples softmax(logits / T) restricted to the legal set,
+        logp is the log-probability of the sampled action under it; T = 0 takes the argmax (ties to the lowest action code,
+        logp 0).  No legal move, or no finite legal logit: RESIGN (4100), logp 0.  The draw walks the legal set in ascending
+        action code, not in the order of legal_actions().  u32: optional int32 / uint32 [N] random words; by default Philox on
+        the env's key (counter: global env id, episode, step in episode, 3 + side to move is black), so sharding is invisible
+        and a clone draws differently from its source.  A pure read: no state, statistic or mask output changes.  With
+        opponent="external" it samples for the bot too once a step has left F_BOT_PENDING (feed the result to bot_ply)."""
+        N = self.num_envs
+        if not isinstance(logits, torch.Tensor) or not logits.is_cuda or logits.device != self.device:
+            raise ValueError("sample_policy: logits must be a cuda tensor on %s" % self.device)
+        if logits.dtype not in (torch.float32, torch.bfloat16):
+            raise ValueError("sample_policy: logits must be float32 or bfloat16, got %s" % logits.dtype)
+        if logits.dim() != 2 or logits.shape[0] != N or logits.shape[1] < self.num_actions:
+            raise ValueError("sample_policy: logits must have shape [%d, >= %d], got %s" % (N, self.num_actions, list(logits.shape)))
+        row_stride = logits.stride(0) if N > 1 else max(logits.stride(0), logits.shape[1])
+        if logits.stride(1) != 1 or row_stride < self.num_actions:
+            raise ValueError("sample_policy: logits need last-dim stride 1 and a row stride >= %d, got strides %s"
+                             % (self.num_actions, list(logits.stride())))
+        temperature = float(temperature)
+        if not (0.0 <= temperature < float("inf")):
+            raise ValueError("sample_policy: temperature must be finite and >= 0, got %r" % temperature)
+        dtype = 0 if logits.dtype == torch.float32 else 1  # GCB_DT_F32 / GCB_DT_BF16
+        u = None
+        if u32 is not None:
+            u = torch.as_tensor(u32, device=self.device)
+            if tuple(u.shape) != (N,):
+                raise ValueError("sample_policy: u32 must have shape [%d], got %s" % (N, list(u.shape)))
+            if u.dtype not in (torch.int32, torch.uint32):
+                u = u.to(torch.int64).to(torch.int32)
+            u = u.contiguous()
+        with torch.cuda.device(self.device):
+            actions = torch.empty(N, dtype=torch.int32, device=self.device)
+            logp = torch.empty(N, dtype=torch.float32, device=self.device)
+            check(_lib.lib().gcb_env_sample_policy(self._h, C.c_void_p(logits.data_ptr()), dtype, row_stride, temperature,
+                                                   C.c_void_p(u.data_ptr()) if u is not None else None,
+                                                   C.c_void_p(actions.data_ptr()), C.c_void_p(logp.data_ptr()), _stream_ptr()))
+        return actions, logp
+
+    def step_policy(self, logits, temperature=1.0):
+        """sample_policy(logits, temperature) followed by step() of the sampled actions on the same stream, with no host
+        synchronisation in between.  -> (actions, logp, reward, done, flags)"""
+        actions, logp = self.sample_policy(logits, temperature)
+        reward, done, flags = self.step(actions)
+        return actions, logp, reward, done, flags
+
     # ------------------------------------------------------------------ stepping (host buffers, copies inside)
     def step_host(self, actions, reward=None, done=None, flags=None):
         """numpy in / numpy out through gcb_env_step_host (H2D + kernel + D2H inside the call)."""

@@ -22,6 +22,8 @@
 //                                            table: {key, generation << 2 | count}; slot = key bits, linear probing;
 //                                            one 16-byte entry read and written per ply
 #pragma once
+#include <math.h>
+
 #include "chess_core.cuh"
 
 #if !defined(__CUDACC__)
@@ -52,8 +54,9 @@ __device__ unsigned long long g_violations = 0ULL;
 #endif
 // CHK_CLONE_INDEX: a clone index >= the source's env count (the row is left alone in both builds); CHK_CLONE_ALIAS: a clone
 // destination row that is also the source row of some destination of the same call
+// CHK_POLICY_INDEX: a policy sample (gcb_env_sample_policy) that would read a logit column >= 4101 or an env row >= N
 enum { CHK_STAT_ROW = 0, CHK_ENV_INDEX = 1, CHK_SLOT_INDEX = 2, CHK_REP_INDEX = 3, CHK_IO_INDEX = 4, CHK_LIST_INDEX = 5,
-       CHK_CLONE_INDEX = 6, CHK_CLONE_ALIAS = 7 };
+       CHK_CLONE_INDEX = 6, CHK_CLONE_ALIAS = 7, CHK_POLICY_INDEX = 8 };
 
 // The resident state is touched once per step: stream it past L1 (ld.global.cs / st.global.cs, evict-first) so that
 // the geometry tables the generation hammers stay L1-resident.
@@ -160,6 +163,12 @@ GCB_HD u64 pack_meta(const EnvRegs& s) {
 
 GCB_HD bool stm_checked(const EnvRegs& s) { return (s.chk >> s.stm_black) & 1u; }
 GCB_HD u64 stm_pieces(const EnvRegs& s) { return s.stm_black ? (bb_occ(s.b) & ~s.b.w) : s.b.w; }
+GCB_HD u32 castle_word(const EnvRegs& s) {  // castle bits of meta -> bit (action - 4096)
+    u32 c = 0;
+    if (s.castle & 1u) c |= 1u << (castle_action(!s.stm_black, 0) - 4096);
+    if (s.castle & 2u) c |= 1u << (castle_action(!s.stm_black, 1) - 4096);
+    return c;
+}
 
 // piece slots of env e in the resident array (slot r of env e at tgt[r*N + e]: coalesced when a warp reads slot r).
 // The per-piece target counts of the first 16 slots go to 16 bytes of scratch (shared memory in the kernel: one
@@ -926,4 +935,107 @@ GCB_HD void env_export_one(const EnvView& v, int e, int8_t* board, int32_t* info
         info[7] = s.done, info[8] = s.move_count, info[9] = s.n_legal, info[10] = (int)v.episode[e], info[11] = s.step;
         info[12] = s.hist_len, info[13] = (int)s.castle, info[14] = s.pending, info[15] = 0;
     }
+}
+
+// ---- Policy sampling (gcb_env_sample_policy): one legal action of the side to move per env, drawn from caller logits.
+// L = the resident legal set of env e (slot r of the r-th own piece, plus the castle bits: what gcb_env_legal_bitmask
+// exports) in ascending ACTION CODE -- from-square, then to-square, then 4096..4099.  That is the order the slots give for
+// free, not the reference's list order.  Only the logits of L are read.  With temperature T > 0: z_a = x_a / T,
+// m = max z, w_a = exp(z_a - m), Z = sum w; the action is the first a of L whose inclusive prefix sum of w exceeds u * Z
+// (policy_u), or the last a with w_a > 0 if rounding leaves none; logp = z_a - m - log Z.  T == 0: the argmax of x over L,
+// ties to the lowest code, logp = 0.  A legal entry of -inf is never chosen; no legal move or no finite legal entry gives
+// RESIGN with logp 0.  Below: the pieces the kernel (k_env_policy_sample) and the serial form share.
+#if defined(__CUDA_ARCH__)
+#define GCB_LDG(p) __ldg(p)
+#else
+#define GCB_LDG(p) (*(p))
+#endif
+GCB_HD float gcb_bits_to_float(u32 x) {
+#if defined(__CUDA_ARCH__)
+    return __uint_as_float(x);
+#else
+    float f;
+    __builtin_memcpy(&f, &x, 4);
+    return f;
+#endif
+}
+// logit a of a row; DT 0 = fp32, 1 = bf16 (GCB_DT_F32 / GCB_DT_BF16), widened exactly: a bf16 is the high half of an fp32
+template <int DT>
+GCB_HD float policy_logit(const void* row, int a) {
+    GCB_CHK((unsigned)a < 4101u, CHK_POLICY_INDEX);
+    if (DT == 1) return gcb_bits_to_float((u32)GCB_LDG(reinterpret_cast<const uint16_t*>(row) + a) << 16);
+    return GCB_LDG(reinterpret_cast<const float*>(row) + a);
+}
+template <int DT>
+GCB_HD const void* policy_row(const void* logits, long long row_stride, int e) {
+    return reinterpret_cast<const char*>(logits) + (size_t)e * (size_t)row_stride * (DT == 1 ? 2u : 4u);
+}
+// the draw u in (0, 1] of a random word: (word >> 8) * 2^-24 + 2^-25 in fp32 -- exact while word >> 8 < 2^23, rounded to
+// nearest even above (the top value rounds to 1.0, which no prefix sum exceeds); one rounding, the same on host and device
+GCB_HD float policy_u(u32 word) { return (float)(word >> 8) * 5.9604644775390625e-08f + 2.98023223876953125e-08f; }
+// the default random word: Philox on the env's key, counter (global env id, episode, step in episode, 3 + side to move is
+// black) -- purposes 0-2 are the step's draws, and the side to move keeps the agent's and an external bot's draws apart
+GCB_HD u32 policy_word(const EnvView& v, int e, const EnvRegs& s, u32 ep) {
+    return philox_draw(v.seed, v.env_offset + (u32)e, ep, (u32)s.step, 3u + (u32)s.stm_black);
+}
+// what a sample reads of the state: board, meta, episode counter (plain loads: a step that follows finds them in L2)
+GCB_HD void policy_load(const EnvView& v, int e, EnvRegs& s, u32& ep) {
+    GCB_CHK((unsigned)e < (unsigned)v.N, CHK_POLICY_INDEX);
+    const ulonglong2 a = v.bb01[e], c = v.bb23[e];
+    s.b.t0 = a.x, s.b.t1 = a.y, s.b.t2 = c.x, s.b.w = c.y;
+    unpack_meta(v.meta[e], s);
+    ep = v.episode[e];
+}
+// greedy step: strict > keeps the lowest code of a tie when L is visited in code order; -inf and NaN never win
+GCB_HD void policy_argmax(float x, int a, float& best, int& pick) {
+    if (x > best) best = x, pick = a;
+}
+// f(a) for every a of L in code order; pieces beyond the slots have no resident targets (as in gcb_env_legal_bitmask)
+template <class F>
+GCB_HD void policy_walk(const EnvView& v, int e, const EnvRegs& s, F f) {
+    const TgtSink slots(resident_slots(v, e), nullptr);
+    int r = 0;
+    for (u64 t = stm_pieces(s); t; t &= t - 1, r++) {
+        const int from = gcb_lsb(t);
+        for (u64 T = slots.get(r); T; T &= T - 1) f(from * 64 + gcb_lsb(T));
+    }
+    for (u32 c = castle_word(s); c; c &= c - 1) f(4096 + gcb_lsb((u64)c));
+}
+// The serial form (the host emulation): three walks over L -- max, sum, prefix-sum selection.
+template <int DT>
+GCB_HD void env_policy_sample_one(const EnvView& v, int e, const void* logits, long long row_stride, float temp, const u32* words,
+                                  int32_t* act, float* logp) {
+    EnvRegs s;
+    u32 ep;
+    policy_load(v, e, s, ep);
+    const void* row = policy_row<DT>(logits, row_stride, e);
+    int pick = -1;
+    float lp = 0.f;
+    if (temp == 0.f) {
+        float best = -INFINITY;
+        policy_walk(v, e, s, [&](int a) { policy_argmax(policy_logit<DT>(row, a), a, best, pick); });
+    } else {
+        float m = -INFINITY;
+        policy_walk(v, e, s, [&](int a) {
+            const float z = policy_logit<DT>(row, a) / temp;
+            if (z > m) m = z;
+        });
+        if (m > -INFINITY) {
+            float Z = 0.f;
+            policy_walk(v, e, s, [&](int a) { Z += expf(policy_logit<DT>(row, a) / temp - m); });
+            const float target = policy_u(words ? GCB_LDG(words + e) : policy_word(v, e, s, ep)) * Z;
+            float acc = 0.f, zp = 0.f, zl = 0.f;
+            int last = -1;
+            policy_walk(v, e, s, [&](int a) {
+                const float z = policy_logit<DT>(row, a) / temp, w = expf(z - m);
+                acc += w;
+                if (pick < 0 && acc > target) pick = a, zp = z;
+                if (w > 0.f) last = a, zl = z;
+            });
+            if (pick < 0) pick = last, zp = zl;
+            lp = zp - m - logf(Z);
+        }
+    }
+    act[e] = pick < 0 ? ACT_RESIGN : pick;
+    if (logp) logp[e] = pick < 0 ? 0.f : lp;
 }

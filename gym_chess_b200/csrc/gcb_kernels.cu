@@ -260,12 +260,6 @@ __device__ __forceinline__ void write_bits_rows(u64* __restrict__ out, int strid
         if (cword) GCB_BITS_ST(row + 64, (u64)cword);
     }
 }
-__device__ __forceinline__ u32 castle_word(const EnvRegs& s) {  // castle bits of meta -> bit (action - 4096)
-    u32 c = 0;
-    if (s.castle & 1u) c |= 1u << (castle_action(!s.stm_black, 0) - 4096);
-    if (s.castle & 2u) c |= 1u << (castle_action(!s.stm_black, 1) - 4096);
-    return c;
-}
 
 // One UNIT of step work of one block: the envs [e, ...) of the block's tile run `nsteps` consecutive steps.
 // TILE selects where the piece slots live while the unit runs:
@@ -598,6 +592,152 @@ __global__ void __launch_bounds__(GCB_BLOCK) k_env_legal_bits(EnvView v, u64* __
         }
         if (lane == 0) __stcs(row + 64, (u64)c_p);
     }
+}
+
+// gcb_env_sample_policy, per-env rule in env_core.cuh (policy_*; env_policy_sample_one is the serial form).  A warp takes
+// the 32 envs of its lanes: each thread loads its env's board, meta and random word and stages its piece slots in shared
+// memory (slot-major, coalesced, as in k_env_legal_bits); then the warp samples the 32 envs one after the other with
+// lane = action.  Lane l owns from-squares 2l and 2l+1, so an inclusive warp scan of the lanes' target counts numbers L in
+// code order; in round j lane l decodes action k = 32j + l (owner lane by a 5-step binary search over the scan, target by
+// gcb_select64) and loads that ONE logit, so the ~23 gathers of an env are in flight together.  Three passes over L: max,
+// sum, prefix-sum selection; the first round's logits stay in registers, later rounds re-read theirs.
+// GCB_POLICY_THREAD = 1 builds the measured alternative instead: one thread per env runs the serial form (DESIGN 3.10).
+#ifndef GCB_POLICY_THREAD
+#define GCB_POLICY_THREAD 0
+#endif
+template <int DT>
+__global__ void __launch_bounds__(GCB_BLOCK) k_env_policy_sample(EnvView v, const void* __restrict__ logits, long long row_stride,
+                                                                 float temp, const u32* __restrict__ words,
+                                                                 int32_t* __restrict__ act, float* __restrict__ logp) {
+    const int e = blockIdx.x * blockDim.x + threadIdx.x, lane = threadIdx.x & 31, wbase = threadIdx.x & ~31;
+#if GCB_POLICY_THREAD
+    if (e < v.N) env_policy_sample_one<DT>(v, e, logits, row_stride, temp, words, act, logp);
+    (void)lane, (void)wbase;
+#else
+    __shared__ u64 s_slots[GCB_SLOTS * GCB_BLOCK];
+    const unsigned FULL = 0xffffffffu;
+    u64 own = 0;
+    u32 cword = 0, word = 0;
+    if (e < v.N) {
+        EnvRegs s;
+        u32 ep;
+        policy_load(v, e, s, ep);
+        own = stm_pieces(s), cword = castle_word(s);
+        if (temp != 0.f) word = words ? __ldg(words + e) : policy_word(v, e, s, ep);
+        const int np = gcb_popc(own);
+        for (int r = 0; r < np && r < GCB_SLOTS; r++) s_slots[r * GCB_BLOCK + threadIdx.x] = __ldcs(v.tgt + (size_t)r * v.N + e);
+    }
+    __syncwarp();
+    const int e0 = e - lane;
+    int my_act = ACT_RESIGN;
+    float my_logp = 0.f;
+#pragma unroll 1
+    for (int p = 0; p < 32 && e0 + p < v.N; p++) {
+        const int ep_ = e0 + p;
+        const u64 own_p = __shfl_sync(FULL, own, p);
+        const u32 cw = __shfl_sync(FULL, cword, p);
+        const void* row = policy_row<DT>(logits, row_stride, ep_);
+        auto slot = [&](int r) -> u64 {
+            return r < GCB_SLOTS ? s_slots[r * GCB_BLOCK + wbase + p] : (r < v.slots ? __ldcs(v.tgt + (size_t)r * v.N + ep_) : 0ULL);
+        };
+        const int sqa = 2 * lane, ra = gcb_popc(own_p & ((1ULL << sqa) - 1));
+        const bool ha = (own_p >> sqa) & 1ULL, hb = (own_p >> (sqa + 1)) & 1ULL;
+        const u64 Ta = ha ? slot(ra) : 0ULL, Tb = hb ? slot(ra + (int)ha) : 0ULL;
+        const int ca = gcb_popc(Ta), c = ca + gcb_popc(Tb);
+        int incl = c;
+#pragma unroll
+        for (int d = 1; d < 32; d <<= 1) {
+            const int t = __shfl_up_sync(FULL, incl, d);
+            if (lane >= d) incl += t;
+        }
+        const int nsq = __shfl_sync(FULL, incl, 31), n = nsq + gcb_popc((u64)cw);
+        // the code of action k of L (all 32 lanes call it; -1 for k >= n)
+        auto code_at = [&](int k) -> int {
+            int pos = 0;  // the owner lane: the number of lanes whose inclusive count is <= k
+#pragma unroll
+            for (int b = 16; b; b >>= 1)
+                if (__shfl_sync(FULL, incl, pos + b - 1) <= k) pos += b;
+            const int excl = __shfl_sync(FULL, incl - c, pos), oca = __shfl_sync(FULL, ca, pos);
+            const u64 oTa = __shfl_sync(FULL, Ta, pos), oTb = __shfl_sync(FULL, Tb, pos);
+            if (k < nsq) {
+                const int i = k - excl;
+                return i < oca ? 128 * pos + gcb_select64(oTa, i) : 128 * pos + 64 + gcb_select64(oTb, i - oca);
+            }
+            return k < n ? 4096 + gcb_select64((u64)cw, k - nsq) : -1;
+        };
+        const int a0 = code_at(lane);
+        int pick = -1;
+        float lp = 0.f;
+        if (temp == 0.f) {
+            float best = -INFINITY;
+            if (a0 >= 0) policy_argmax(policy_logit<DT>(row, a0), a0, best, pick);
+            for (int base = 32; base < n; base += 32) {
+                const int a = code_at(base + lane);
+                if (a >= 0) policy_argmax(policy_logit<DT>(row, a), a, best, pick);
+            }
+#pragma unroll
+            for (int d = 16; d; d >>= 1) {  // warp argmax: the larger logit, then the lower code
+                const float ob = __shfl_xor_sync(FULL, best, d);
+                const int oi = __shfl_xor_sync(FULL, pick, d);
+                if (oi >= 0 && (pick < 0 || ob > best || (ob == best && oi < pick))) best = ob, pick = oi;
+            }
+        } else {
+            const float z0 = a0 >= 0 ? policy_logit<DT>(row, a0) / temp : 0.f;
+            float m = a0 >= 0 && z0 > -INFINITY ? z0 : -INFINITY;
+            for (int base = 32; base < n; base += 32) {
+                const int a = code_at(base + lane);
+                if (a >= 0) {
+                    const float z = policy_logit<DT>(row, a) / temp;
+                    if (z > m) m = z;
+                }
+            }
+#pragma unroll
+            for (int d = 16; d; d >>= 1) {
+                const float o = __shfl_xor_sync(FULL, m, d);
+                if (o > m) m = o;
+            }
+            if (m > -INFINITY) {
+                float Z = a0 >= 0 ? expf(z0 - m) : 0.f;
+                for (int base = 32; base < n; base += 32) {
+                    const int a = code_at(base + lane);
+                    if (a >= 0) Z += expf(policy_logit<DT>(row, a) / temp - m);
+                }
+#pragma unroll
+                for (int d = 16; d; d >>= 1) Z += __shfl_xor_sync(FULL, Z, d);
+                Z = __shfl_sync(FULL, Z, 0);  // (lanes may round the butterfly differently: lane 0's sum for all)
+                const float target = policy_u(__shfl_sync(FULL, word, p)) * Z;
+                float carry = 0.f, zp = 0.f;
+                int last = -1;
+                for (int base = 0; base < n && pick < 0; base += 32) {
+                    const int a = base == 0 ? a0 : code_at(base + lane);
+                    const float z = base == 0 ? z0 : (a >= 0 ? policy_logit<DT>(row, a) / temp : 0.f);
+                    const float w = a >= 0 ? expf(z - m) : 0.f;
+                    float pre = w;
+#pragma unroll
+                    for (int d = 1; d < 32; d <<= 1) {
+                        const float t = __shfl_up_sync(FULL, pre, d);
+                        if (lane >= d) pre += t;
+                    }
+                    pre += carry;
+                    const unsigned hit = __ballot_sync(FULL, a >= 0 && pre > target), pos = __ballot_sync(FULL, a >= 0 && w > 0.f);
+                    if (hit) {
+                        pick = __shfl_sync(FULL, a, __ffs(hit) - 1), zp = __shfl_sync(FULL, z, __ffs(hit) - 1);
+                    } else if (pos) {  // (the last a with w > 0 so far: the pick if rounding leaves no prefix sum above target)
+                        last = __shfl_sync(FULL, a, 31 - __clz(pos)), zp = __shfl_sync(FULL, z, 31 - __clz(pos));
+                    }
+                    carry = __shfl_sync(FULL, pre, 31);
+                }
+                if (pick < 0) pick = last;
+                lp = zp - m - logf(Z);
+            }
+        }
+        if (lane == p) my_act = pick < 0 ? ACT_RESIGN : pick, my_logp = pick < 0 ? 0.f : lp;
+    }
+    if (e < v.N) {
+        act[e] = my_act;
+        if (logp) logp[e] = my_logp;
+    }
+#endif
 }
 
 // ------------------------------------------------------------------------------------------------ host side
@@ -1396,6 +1536,22 @@ extern "C" int gcb_env_legal_bitmask(gcb_env* env, uint64_t* d_bits, int stride_
     ENV_CHECK(env);
     if (!d_bits || stride_words < 65) return fail(GCB_E_ARG, "gcb_env_legal_bitmask", "null pointer or stride_words < 65");
     k_env_legal_bits<<<grid_for(env->v.N), GCB_BLOCK, 0, (cudaStream_t)stream>>>(env->v, reinterpret_cast<u64*>(d_bits), stride_words, 0, env->v.N);
+    LAUNCHED();
+    return GCB_OK;
+}
+
+extern "C" int gcb_env_sample_policy(const gcb_env* env, const void* d_logits, int dtype, int64_t row_stride, float temperature,
+                                     const uint32_t* d_u32, int32_t* d_actions, float* d_logp, void* stream) {
+    ENV_CHECK(env);
+    if (dtype != GCB_DT_F32 && dtype != GCB_DT_BF16) return fail(GCB_E_ARG, "gcb_env_sample_policy", "dtype must be GCB_DT_F32 or GCB_DT_BF16");
+    if (row_stride < 4101) return fail(GCB_E_ARG, "gcb_env_sample_policy", "row_stride < 4101");
+    if (!(temperature >= 0.f && temperature < INFINITY)) return fail(GCB_E_ARG, "gcb_env_sample_policy", "temperature must be finite and >= 0");
+    if (!d_logits || !d_actions) return fail(GCB_E_ARG, "gcb_env_sample_policy", "null logits or actions");
+    const cudaStream_t s = (cudaStream_t)stream;
+    if (dtype == GCB_DT_F32)
+        k_env_policy_sample<0><<<grid_for(env->v.N), GCB_BLOCK, 0, s>>>(env->v, d_logits, (long long)row_stride, temperature, d_u32, d_actions, d_logp);
+    else
+        k_env_policy_sample<1><<<grid_for(env->v.N), GCB_BLOCK, 0, s>>>(env->v, d_logits, (long long)row_stride, temperature, d_u32, d_actions, d_logp);
     LAUNCHED();
     return GCB_OK;
 }

@@ -266,6 +266,38 @@ int gcb_env_step_mask_output(gcb_env *env, uint64_t *d_bits, int stride_words);
  * count.  Like the reference's property, the list is DERIVED on access: the resident form of possible_moves is one
  * 64-bit legal-target set per own piece (gcb_env_piece_slots) and the list is a pure decode of (board, slots). */
 int gcb_env_legal_actions(gcb_env *env, uint16_t *d_actions, int stride, int32_t *d_counts, void *stream);
+
+/* Policy sampling: for every env, one legal action of the SIDE TO MOVE drawn from caller logits over the 4101-way action
+ * space -- the act step of a learned policy, without building a mask.  d_logits [N][row_stride] (device), element type
+ * dtype (GCB_DT_F32 or GCB_DT_BF16), row_stride >= 4101 elements; only the entries of legal actions are read.
+ *   L: the env's resident legal set (what gcb_env_legal_bitmask exports: word `from` = the legal targets of the piece on
+ *      that square, plus the castle bits), ordered by ASCENDING ACTION CODE -- from-square, then to-square, then
+ *      4096..4099.  This is deliberately not the order of gcb_env_legal_actions (the reference's list order): it is the
+ *      order the piece slots give for free, and what np.nonzero of an unpacked bit mask gives.
+ *   temperature T > 0: z_a = x_a / T, m = max_{a in L} z_a, w_a = exp(z_a - m), Z = sum w_a; the draw is
+ *      u = (word >> 8) * 2^-24 + 2^-25 in fp32 (exact for word < 2^31, rounded to nearest even above; the same on every
+ *      device); the action is the first a of L whose inclusive prefix sum of w exceeds u * Z, or the last a with w_a > 0
+ *      if rounding leaves none.  d_logp[e] = z_a - m - log Z (fp32).  Sums run in fp32; their order is unspecified.
+ *   T == 0: greedy -- the argmax of x over L, ties to the lowest code; d_logp = 0 (the log-probability of the degenerate
+ *      distribution that was sampled).
+ *   A legal entry of -inf is never chosen.  When L is empty, or no legal entry is finite, the action is GCB_ACT_RESIGN with
+ *   logp 0 (what gcb_env_step_index plays without a legal move).  +inf or NaN on a legal entry, or an x / T that overflows,
+ *   gives an unspecified legal action or GCB_ACT_RESIGN.
+ *   Random words: d_u32 uint32[N] (device) supplies them; NULL draws Philox4x32-10 on the env's key with counter (global env
+ *   id, episode, step in episode, 3 + side to move is black) -- purposes 0-2 are the step's draws, the side to move keeps an
+ *   agent's and an external bot's draw at the same step apart.  Sharding (env_id_offset) is therefore invisible, and a clone
+ *   (gcb_env_clone) draws differently from its source.
+ * The call only reads the env: no state, statistic or registered mask output changes, and two calls without a step in
+ * between return the same sample.  It samples for whichever side is to move: with opponent 2 (external), after a step
+ * reported GCB_F_BOT_PENDING, that is the bot (feed the result to gcb_env_bot_ply).  An env that is done (auto_reset off)
+ * or has more own pieces than piece slots is sampled from its resident set as it stands, as gcb_env_legal_bitmask exports
+ * it.  d_actions int32[N] (required), d_logp float32[N] (may be NULL).  GCB_E_ARG for a bad dtype, row_stride < 4101, a
+ * negative or non-finite temperature, or a NULL d_logits / d_actions.  The CHECKED build records a logit column >= 4101 or
+ * an env row >= N as CHK_POLICY_INDEX (bit 8 of gcb_debug_violations). */
+#define GCB_DT_F32 0
+#define GCB_DT_BF16 1
+int gcb_env_sample_policy(const gcb_env *env, const void *d_logits, int dtype, int64_t row_stride, float temperature,
+                          const uint32_t *d_u32, int32_t *d_actions, float *d_logp, void *stream);
 /* zero-copy views of the resident state: slots uint64[n_slots][N] (slot r of env e at [r][e] = legal targets of the
  * r-th piece, in ascending square order, of the side to move); positions (player/rights are NULL: they live in meta) */
 int gcb_env_piece_slots(gcb_env *env, uint64_t **d_slots, int32_t *n_slots);
