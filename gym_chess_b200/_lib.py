@@ -126,6 +126,7 @@ SIGNATURES = {
     "gcb_env_step_mask_output": (i32, [vp, vp, i32]),
     "gcb_env_legal_actions": (i32, [vp, vp, i32, vp, vp]),
     "gcb_env_sample_policy": (i32, [vp, vp, i32, C.c_int64, C.c_float, vp, vp, vp, vp]),
+    "gcb_env_encode": (i32, [vp, vp, i32, vp, vp]),
     "gcb_env_piece_slots": (i32, [vp, C.POINTER(vp), C.POINTER(C.c_int32)]),
     "gcb_env_positions": (i32, [vp, C.POINTER(Positions)]),
     "gcb_env_snapshot_bytes": (i32, [vp, C.POINTER(C.c_uint64)]),

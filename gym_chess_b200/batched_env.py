@@ -24,6 +24,12 @@ STAT_NAMES = ("steps", "plies", "episodes", "mates", "repetitions", "caps", "wed
 INFO_NAMES = ("current_player", "white_king_castle_is_possible", "white_queen_castle_is_possible",
               "black_king_castle_is_possible", "black_queen_castle_is_possible", "white_king_is_checked",
               "black_king_is_checked", "done", "move_count", "n_legal", "episode", "step_in_episode", "hist_len", "castles", "bot_pending")
+# the 19 planes of encode(), in order
+OBS_PLANE_NAMES = ("white_king", "white_queen", "white_rook", "white_bishop", "white_knight", "white_pawn",
+                   "black_king", "black_queen", "black_rook", "black_bishop", "black_knight", "black_pawn", "black_to_move",
+                   "white_king_castle_is_possible", "white_queen_castle_is_possible", "black_king_castle_is_possible",
+                   "black_queen_castle_is_possible", "repeated_once", "repeated_twice")
+_ENCODE_DTYPES = {torch.float32: 0, torch.bfloat16: 1, torch.uint8: 2}  # GCB_DT_F32 / GCB_DT_BF16 / GCB_DT_U8
 
 
 class _DevArray:
@@ -331,6 +337,40 @@ class BatchedChessEnv:
             t = torch.empty((self.num_envs, 16), dtype=torch.int32, device=self.device)
             check(_lib.lib().gcb_env_export(self._h, None, C.c_void_p(t.data_ptr()), _stream_ptr()))
         return t
+
+    def encode(self, dtype=torch.float32, out=None):
+        """The network input of every env: [N, 19, 8, 8] binary planes (OBS_PLANE_NAMES) in float32, bfloat16 or uint8,
+        square [row, col] with row 0 = rank 8 (the orientation of observe() and of the action codes, not mirrored for the
+        side to move).  Planes 0-5 White K Q R B N P, 6-11 Black K Q R B N P, 12 Black to move, 13-16 the castle flags
+        wk wq bk bq (info_tensor() columns 1-4), 17 the board has occurred at least once and 18 at least twice as the pre-move
+        board of a ply of this episode -- with 18 set, the next ply ends the episode with F_REPETITION.  The count comes from
+        the env's repetition table, so it misses a repetition exactly where the step does (a window beyond history_cap, a
+        64-bit key collision).  out: a contiguous, 16-byte aligned tensor of this shape and dtype on the env's device (e.g.
+        buf[t] of a [T, N, 19, 8, 8] rollout buffer), written in place and returned.  A pure read of the env: no state,
+        statistic or mask output changes."""
+        if dtype not in _ENCODE_DTYPES:
+            raise ValueError("encode: dtype must be torch.float32, torch.bfloat16 or torch.uint8, got %r" % (dtype,))
+        shape = (self.num_envs, 19, 8, 8)
+        if out is None:
+            with torch.cuda.device(self.device):
+                out = torch.empty(shape, dtype=dtype, device=self.device)
+        elif not isinstance(out, torch.Tensor) or not out.is_cuda or out.device != self.device:
+            raise ValueError("encode: out must be a cuda tensor on %s" % self.device)
+        elif out.dtype != dtype or tuple(out.shape) != shape:
+            raise ValueError("encode: out must be %s %s, got %s %s" % (dtype, list(shape), out.dtype, list(out.shape)))
+        elif not out.is_contiguous() or out.data_ptr() % 16:
+            raise ValueError("encode: out must be contiguous and 16-byte aligned")
+        with torch.cuda.device(self.device):
+            check(_lib.lib().gcb_env_encode(self._h, C.c_void_p(out.data_ptr()), _ENCODE_DTYPES[dtype], None, _stream_ptr()))
+        return out
+
+    def repetition_count(self):
+        """uint8 [N]: how often the current board has occurred as the pre-move board of a ply of this episode, saturated at
+        2 (= planes 17 + 18 of encode(); 2: the next ply ends the episode with F_REPETITION).  A pure read."""
+        with torch.cuda.device(self.device):
+            rep = torch.empty(self.num_envs, dtype=torch.uint8, device=self.device)
+            check(_lib.lib().gcb_env_encode(self._h, None, 0, C.c_void_p(rep.data_ptr()), _stream_ptr()))
+        return rep
 
     def legal_actions(self, stride=None):
         """(legal int16-viewed uint16 [N, stride], n_legal int32 [N]) = possible_actions in the reference's order,

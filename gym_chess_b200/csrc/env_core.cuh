@@ -55,8 +55,9 @@ __device__ unsigned long long g_violations = 0ULL;
 // CHK_CLONE_INDEX: a clone index >= the source's env count (the row is left alone in both builds); CHK_CLONE_ALIAS: a clone
 // destination row that is also the source row of some destination of the same call
 // CHK_POLICY_INDEX: a policy sample (gcb_env_sample_policy) that would read a logit column >= 4101 or an env row >= N
+// CHK_ENCODE_INDEX: an encode (gcb_env_encode) that would read an env row >= N or write a plane element beyond [N][19][64]
 enum { CHK_STAT_ROW = 0, CHK_ENV_INDEX = 1, CHK_SLOT_INDEX = 2, CHK_REP_INDEX = 3, CHK_IO_INDEX = 4, CHK_LIST_INDEX = 5,
-       CHK_CLONE_INDEX = 6, CHK_CLONE_ALIAS = 7, CHK_POLICY_INDEX = 8 };
+       CHK_CLONE_INDEX = 6, CHK_CLONE_ALIAS = 7, CHK_POLICY_INDEX = 8, CHK_ENCODE_INDEX = 9 };
 
 // The resident state is touched once per step: stream it past L1 (ld.global.cs / st.global.cs, evict-first) so that
 // the geometry tables the generation hammers stay L1-resident.
@@ -1038,4 +1039,56 @@ GCB_HD void env_policy_sample_one(const EnvView& v, int e, const void* logits, l
     }
     act[e] = pick < 0 ? ACT_RESIGN : pick;
     if (logp) logp[e] = pick < 0 ? 0.f : lp;
+}
+
+// ---- Network input (gcb_env_encode): 19 binary planes of 8 x 8 per env, square sq = row * 8 + col (row 0 = rank 8), as
+// 64-bit masks (bit sq of mask c = element [c][sq]): 0-5 White K Q R B N P, 6-11 Black K Q R B N P, 12 Black to move,
+// 13-16 castle flags wk wq bk bq, 17 the board has occurred >= 1 time and 18 >= 2 times as the pre-move board of a ply of
+// this episode.  The count is the repetition table's, probed with the board-only key the step uses, without inserting:
+// rep_lookup_insert answers "occurrences including this ply" = stored count + 1, and saturates at 3.  A window that has
+// outgrown the table (its overflow branch answers 1) or a key collision can miss a repetition here exactly as in the step.
+enum { OBS_PLANES = 19 };
+GCB_HD void env_encode_masks(const EnvView& v, int e, u64* m, int* rep) {
+    GCB_CHK((unsigned)e < (unsigned)v.N, CHK_ENCODE_INDEX);
+    EnvRegs s;
+    const ulonglong2 a = v.bb01[e], c = v.bb23[e];
+    s.b.t0 = a.x, s.b.t1 = a.y, s.b.t2 = c.x, s.b.w = c.y;
+    unpack_meta(v.meta[e], s);
+    const u64 white = s.b.w, black = bb_occ(s.b) & ~s.b.w;
+    const u64 kind[6] = {bb_kings(s.b), bb_queens(s.b), bb_rooks(s.b), bb_bishops(s.b), bb_knights(s.b), bb_pawns(s.b)};
+    for (int k = 0; k < 6; k++) m[k] = kind[k] & white, m[6 + k] = kind[k] & black;
+    m[12] = s.stm_black ? ~0ULL : 0ULL;
+    for (int k = 0; k < 4; k++) m[13 + k] = (s.rights >> k) & 1u ? ~0ULL : 0ULL;  // RT_WK, RT_WQ, RT_BK, RT_BQ
+    int n = 0;
+    if (s.hist_len != 0) {  // an empty window holds no live entry: nothing to read
+        s.zk = v.zkey[e], s.gen = v.gen[e];
+        StepStats local;
+        local.clear();
+        n = rep_lookup_insert(v, e, s, hist_key(s.zk), /*insert=*/false, local) - 1;
+    }
+    m[17] = n >= 1 ? ~0ULL : 0ULL;
+    m[18] = n >= 2 ? ~0ULL : 0ULL;
+    *rep = n;
+}
+// element values: DT 0 = fp32, 1 = bf16 (as its 16-bit pattern), 2 = uint8 (GCB_DT_F32 / GCB_DT_BF16 / GCB_DT_U8)
+template <int DT> struct EncodeElem { typedef float type; };
+template <> struct EncodeElem<1> { typedef uint16_t type; };
+template <> struct EncodeElem<2> { typedef uint8_t type; };
+template <int DT>
+GCB_HD typename EncodeElem<DT>::type encode_value(u32 bit) {
+    if (DT == 0) return bit ? 1.0f : 0.0f;
+    return (typename EncodeElem<DT>::type)(DT == 1 ? bit * 0x3F80u : bit);  // bf16 1.0 = 0x3F80
+}
+// The serial form (the host emulation): env e's masks expanded into its row planes[e][19][64]; rep_out[e] (either may be NULL)
+template <int DT>
+GCB_HD void env_encode_one(const EnvView& v, int e, typename EncodeElem<DT>::type* planes, uint8_t* rep_out) {
+    u64 m[OBS_PLANES];
+    int rep;
+    env_encode_masks(v, e, m, &rep);
+    if (planes) {
+        typename EncodeElem<DT>::type* row = planes + (size_t)e * OBS_PLANES * 64;
+        for (int c = 0; c < OBS_PLANES; c++)
+            for (int sq = 0; sq < 64; sq++) row[c * 64 + sq] = encode_value<DT>((u32)(m[c] >> sq) & 1u);
+    }
+    if (rep_out) rep_out[e] = (uint8_t)rep;
 }

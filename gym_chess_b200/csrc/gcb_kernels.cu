@@ -740,6 +740,54 @@ __global__ void __launch_bounds__(GCB_BLOCK) k_env_policy_sample(EnvView v, cons
 #endif
 }
 
+// gcb_env_encode, per-env rule in env_core.cuh (env_encode_masks; env_encode_one is the serial form).  The output rows of the
+// 32 envs of a warp are ONE contiguous span of 32 x 19 x 64 elements.  Each lane puts its env's 19 masks into shared memory,
+// env-major, so that mask word w of the warp holds elements [64 w, 64 w + 64) of the span; then the warp writes the span
+// flat, one 16-byte vector per lane per iteration (4 / 8 / 16 elements from one broadcast mask word; a vector never straddles
+// two words), with streaming stores.  A pure write stream: the state it reads is 40 B per env plus the table probe of envs
+// with a non-empty window.
+template <int DT>
+__device__ __forceinline__ uint4 encode_vec(u32 bits) {  // the 16 / 8 / 4 low bits of `bits` -> one 16-byte vector
+    uint4 r;
+    if (DT == 2) {  // bit i of a nibble -> byte i: the copies of the nibble shifted by 7 do not overlap
+        r.x = ((bits & 15u) * 0x204081u) & 0x01010101u, r.y = (((bits >> 4) & 15u) * 0x204081u) & 0x01010101u;
+        r.z = (((bits >> 8) & 15u) * 0x204081u) & 0x01010101u, r.w = ((bits >> 12) * 0x204081u) & 0x01010101u;
+    } else if (DT == 1) {  // two bf16 per word, 1.0 = 0x3F80
+        r.x = (bits & 1u) * 0x3F80u + ((bits >> 1) & 1u) * 0x3F800000u, r.y = ((bits >> 2) & 1u) * 0x3F80u + ((bits >> 3) & 1u) * 0x3F800000u;
+        r.z = ((bits >> 4) & 1u) * 0x3F80u + ((bits >> 5) & 1u) * 0x3F800000u, r.w = ((bits >> 6) & 1u) * 0x3F80u + (bits >> 7) * 0x3F800000u;
+    } else {  // fp32 1.0 = 0x3F800000
+        r.x = (bits & 1u) * 0x3F800000u, r.y = ((bits >> 1) & 1u) * 0x3F800000u;
+        r.z = ((bits >> 2) & 1u) * 0x3F800000u, r.w = (bits >> 3) * 0x3F800000u;
+    }
+    return r;
+}
+template <int DT>
+__global__ void __launch_bounds__(GCB_BLOCK) k_env_encode(EnvView v, void* __restrict__ planes, uint8_t* __restrict__ rep_out) {
+    __shared__ u64 s_masks[GCB_BLOCK * OBS_PLANES];
+    const int e = blockIdx.x * blockDim.x + threadIdx.x, lane = threadIdx.x & 31;
+    u64* const wm = s_masks + (threadIdx.x & ~31) * OBS_PLANES;
+    if (e < v.N) {
+        u64 m[OBS_PLANES];
+        int rep;
+        env_encode_masks(v, e, m, &rep);
+#pragma unroll
+        for (int c = 0; c < OBS_PLANES; c++) wm[lane * OBS_PLANES + c] = m[c];
+        if (rep_out) rep_out[e] = (uint8_t)rep;
+    }
+    if (!planes) return;
+    __syncwarp();
+    constexpr int V = 16 / (int)sizeof(typename EncodeElem<DT>::type), PER_ENV = OBS_PLANES * 64 / V;
+    const int e0 = e - lane, nvec = min(32, v.N - e0) * PER_ENV;  // a partial last warp writes only its envs' rows
+    uint4* const out = reinterpret_cast<uint4*>(planes) + (size_t)e0 * PER_ENV;
+#pragma unroll 4
+    for (int j = lane; j < nvec; j += 32) {
+        const int k = j * V;
+        const u32 bits = (u32)(wm[k >> 6] >> (k & 63)) & ((1u << V) - 1u);
+        GCB_CHK((size_t)e0 * PER_ENV + (size_t)j < (size_t)v.N * PER_ENV, CHK_ENCODE_INDEX);
+        __stcs(out + j, encode_vec<DT>(bits));
+    }
+}
+
 // ------------------------------------------------------------------------------------------------ host side
 static int need_gpu() {
     int n = 0;
@@ -1552,6 +1600,20 @@ extern "C" int gcb_env_sample_policy(const gcb_env* env, const void* d_logits, i
         k_env_policy_sample<0><<<grid_for(env->v.N), GCB_BLOCK, 0, s>>>(env->v, d_logits, (long long)row_stride, temperature, d_u32, d_actions, d_logp);
     else
         k_env_policy_sample<1><<<grid_for(env->v.N), GCB_BLOCK, 0, s>>>(env->v, d_logits, (long long)row_stride, temperature, d_u32, d_actions, d_logp);
+    LAUNCHED();
+    return GCB_OK;
+}
+
+extern "C" int gcb_env_encode(const gcb_env* env, void* d_planes, int dtype, uint8_t* d_rep, void* stream) {
+    ENV_CHECK(env);
+    if (dtype != GCB_DT_F32 && dtype != GCB_DT_BF16 && dtype != GCB_DT_U8)
+        return fail(GCB_E_ARG, "gcb_env_encode", "dtype must be GCB_DT_F32, GCB_DT_BF16 or GCB_DT_U8");
+    if (!d_planes && !d_rep) return fail(GCB_E_ARG, "gcb_env_encode", "d_planes and d_rep are both NULL");
+    if (reinterpret_cast<uintptr_t>(d_planes) & 15u) return fail(GCB_E_ARG, "gcb_env_encode", "d_planes is not 16-byte aligned");
+    const cudaStream_t s = (cudaStream_t)stream;
+    if (dtype == GCB_DT_F32) k_env_encode<0><<<grid_for(env->v.N), GCB_BLOCK, 0, s>>>(env->v, d_planes, d_rep);
+    else if (dtype == GCB_DT_BF16) k_env_encode<1><<<grid_for(env->v.N), GCB_BLOCK, 0, s>>>(env->v, d_planes, d_rep);
+    else k_env_encode<2><<<grid_for(env->v.N), GCB_BLOCK, 0, s>>>(env->v, d_planes, d_rep);
     LAUNCHED();
     return GCB_OK;
 }

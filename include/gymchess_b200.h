@@ -296,8 +296,35 @@ int gcb_env_legal_actions(gcb_env *env, uint16_t *d_actions, int stride, int32_t
  * an env row >= N as CHK_POLICY_INDEX (bit 8 of gcb_debug_violations). */
 #define GCB_DT_F32 0
 #define GCB_DT_BF16 1
+#define GCB_DT_U8 2 /* gcb_env_encode only */
 int gcb_env_sample_policy(const gcb_env *env, const void *d_logits, int dtype, int64_t row_stride, float temperature,
                           const uint32_t *d_u32, int32_t *d_actions, float *d_logp, void *stream);
+
+/* Network input: every env's state as GCB_OBS_PLANES = 19 binary planes of 8 x 8.  d_planes [N][19][64] of dtype
+ * (GCB_DT_F32, GCB_DT_BF16 or GCB_DT_U8; every element is 0 or 1), contiguous, 16-byte aligned (device).  Element
+ * [e][c][sq] belongs to square sq = row * 8 + col, row 0 = rank 8: the orientation of the board export and of the action
+ * codes (absolute, not mirrored for the side to move).
+ *   planes 0-5    White K, Q, R, B, N, P (wire codes 1..6)
+ *   planes 6-11   Black K, Q, R, B, N, P
+ *   plane 12      all ones iff Black is to move
+ *   planes 13-16  all ones iff the castle flag is set: wk, wq, bk, bq (the `rights` field, export info columns 1-4)
+ *   plane 17      all ones iff the current board has occurred AT LEAST ONCE as the pre-move board of a ply of this episode
+ *                 (the reference's saved_boards[encode_board(board)] >= 1, chess_v2.py:404-407)
+ *   plane 18      all ones iff it has occurred AT LEAST TWICE: the next ply played from this board ends the episode with
+ *                 GCB_F_REPETITION
+ * d_rep uint8[N] (device) receives that count saturated at 2, i.e. plane 17 + plane 18.  Either output may be NULL, not both.
+ * The count comes from the env's repetition table with the board-only key the step itself uses, so it means exactly what the
+ * next step will see -- including the step's blind spots: a window that has outgrown history_cap (statistic hist_overflow)
+ * or a 64-bit Zobrist key collision can miss a repetition here just as it can in the step.  Only envs with a non-empty
+ * window (export info column hist_len != 0) read the table.
+ * The call is a pure read: no state, statistic, Philox counter or registered mask output changes, and two calls without a
+ * step in between write identical bytes.  It encodes whatever each env holds: the side to move (the bot, while an external
+ * env owes a ply), a done env (auto_reset off), a fresh import (counts 0) and a clone (its source's table: it encodes
+ * exactly like its source).  GCB_E_ARG for a bad dtype, both outputs NULL, or a d_planes that is not 16-byte aligned.
+ * Enqueued on `stream`.  The CHECKED build records an env row >= N or a plane element beyond [N][19][64] as
+ * CHK_ENCODE_INDEX (bit 9 of gcb_debug_violations). */
+#define GCB_OBS_PLANES 19
+int gcb_env_encode(const gcb_env *env, void *d_planes, int dtype, uint8_t *d_rep, void *stream);
 /* zero-copy views of the resident state: slots uint64[n_slots][N] (slot r of env e at [r][e] = legal targets of the
  * r-th piece, in ascending square order, of the side to move); positions (player/rights are NULL: they live in meta) */
 int gcb_env_piece_slots(gcb_env *env, uint64_t **d_slots, int32_t *n_slots);
