@@ -875,6 +875,27 @@ GCB_HD void make_template_one(int i, const int8_t* boards, ulonglong2* bb01, ulo
     zkey[i] = s.zk;
 }
 
+// Host set-up that gcb_env_create and the host emulation share.  The start position (DEFAULT_BOARD): the template when no
+// initial boards are given.
+static const int8_t kDefaultBoard[64] = {-3, -5, -4, -2, -1, -4, -5, -3, -6, -6, -6, -6, -6, -6, -6, -6, 0, 0, 0, 0, 0, 0,
+                                         0,  0,  0,  0,  0,  0,  0,  0,  0,  0,  0,  0,  0,  0,  0,  0,  0, 0, 0, 0, 0, 0,
+                                         0,  0,  0,  0,  6,  6,  6,  6,  6,  6,  6,  6,  3,  5,  4,  2,  1, 4, 5, 3};
+// The automatic piece-slot count (piece_slots = 0): one slot per own piece of the side to move -- the most pieces either side
+// has on any template, at least 16.  Piece counts never grow (no promotion in play, Q1).
+static inline int auto_piece_slots(int n_templates, const int8_t* template_boards) {
+    int need = 16;
+    for (int t = 0; t < n_templates && template_boards; t++) {
+        int w = 0, bl = 0;
+        for (int sq = 0; sq < 64; sq++) {
+            int8_t p = template_boards[(size_t)t * 64 + sq];
+            w += p > 0, bl += p < 0;
+        }
+        need = need < w ? w : need;
+        need = need < bl ? bl : need;
+    }
+    return need;
+}
+
 // ordered list -> memory, one uint16 per move at its list position (moves beyond `cap` are dropped, the count is kept)
 struct ListOut {
     uint16_t* out;

@@ -1028,10 +1028,6 @@ static cudaError_t env_alloc(gcb_env* env, const char* name, void** out, size_t 
     return cudaSuccess;
 }
 
-static const int8_t kDefaultBoard[64] = {-3, -5, -4, -2, -1, -4, -5, -3, -6, -6, -6, -6, -6, -6, -6, -6, 0, 0, 0, 0, 0, 0,
-                                         0,  0,  0,  0,  0,  0,  0,  0,  0,  0,  0,  0,  0,  0,  0,  0,  0, 0, 0, 0, 0, 0,
-                                         0,  0,  0,  0,  6,  6,  6,  6,  6,  6,  6,  6,  3,  5,  4,  2,  1, 4, 5, 3};
-
 // single-step launches: with the default 16 piece slots the generation runs on the shared-memory tile (TILE 2)
 template <int MODE>
 static int launch_io(gcb_env* env, StepIO& io, cudaStream_t s) {
@@ -1088,18 +1084,8 @@ extern "C" int gcb_env_create(const gcb_env_config* cfg_in, gcb_env** out) {
     if (int rc = need_gpu()) return rc;
     gcb_env_config cfg = *cfg_in;
     if (cfg.num_envs <= 0) return fail(GCB_E_ARG, "gcb_env_create", "num_envs <= 0");
-    // piece slots: one per own piece of the side to move; piece counts never grow (no promotion in play, Q1)
     {
-        int need = 16;
-        for (int t = 0; t < cfg.n_templates && cfg.template_boards; t++) {
-            int w = 0, bl = 0;
-            for (int sq = 0; sq < 64; sq++) {
-                int8_t p = cfg.template_boards[(size_t)t * 64 + sq];
-                w += p > 0, bl += p < 0;
-            }
-            need = need < w ? w : need;
-            need = need < bl ? bl : need;
-        }
+        const int need = auto_piece_slots(cfg.n_templates, cfg.template_boards);
         if (cfg.piece_slots == 0) cfg.piece_slots = need;
         if (cfg.piece_slots < need || cfg.piece_slots > 64)
             return fail(GCB_E_ARG, "gcb_env_create", "piece_slots must be 0 (auto) or in [max pieces per side, 64]");

@@ -1,7 +1,8 @@
 """ctypes binding of tests/host_emul/host_emul.cpp (TEST INFRASTRUCTURE: the device rules compiled with g++).
 
 Lets `pytest -m "not gpu"` check the bitboard / step logic of gym_chess_b200/csrc/*.cuh against the oracle
-without a GPU.  Never imported by the product package.
+without a GPU, and the per-env clone, policy sampling and the network-input encoder (EmulEnv.clone_from, sample_policy,
+encode: the logic of gcb_env_clone, gcb_env_sample_policy and gcb_env_encode).  Never imported by the product package.
 """
 import ctypes as C
 import os
@@ -13,13 +14,13 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 _SO = os.path.join(_HERE, "libhost_emul.so")
 _CSRC = os.path.join(_HERE, "..", "..", "gym_chess_b200", "csrc")
 _lib = None
+_ENCODE_DTYPES = {np.dtype(np.float32): 0, np.dtype(np.uint16): 1, np.dtype(np.uint8): 2}  # uint16 = bf16 bit patterns
 
 
 def build(force=False):
     srcs = [os.path.join(_HERE, "host_emul.cpp"), os.path.join(_CSRC, "chess_core.cuh"), os.path.join(_CSRC, "env_core.cuh")]
     if force or not os.path.exists(_SO) or os.path.getmtime(_SO) < max(os.path.getmtime(s) for s in srcs):
-        extra = os.environ.get("GCB_EMUL_CFLAGS", "").split()  # e.g. -DGCB_PAIR=1: check a kernel variant's logic on the CPU
-        subprocess.check_call(["g++", "-O2", "-std=c++17", "-fPIC", "-shared", "-Wno-unknown-pragmas"] + extra + ["-o", _SO, srcs[0]])
+        subprocess.check_call(["g++", "-O2", "-std=c++17", "-fPIC", "-shared", "-Wno-unknown-pragmas", "-o", _SO, srcs[0]])
     return _SO
 
 
@@ -43,6 +44,10 @@ def lib():
         L.emul_env_export.argtypes = [vp, vp, vp, vp, C.c_int]
         L.emul_env_import.argtypes = [vp] * 6
         L.emul_env_stats.argtypes = [vp, vp]
+        L.emul_env_piece_slots.argtypes = [vp]
+        L.emul_env_clone.argtypes = [vp] * 3
+        L.emul_env_sample_policy.argtypes = [vp, vp, C.c_int, C.c_longlong, C.c_float, vp, vp, vp]
+        L.emul_env_encode.argtypes = [vp, vp, C.c_int, vp]
         L.emul_pack_result.argtypes = [C.c_int, C.c_int, C.c_uint32]
         L.emul_pack_result.restype = C.c_uint16
         _lib = L
@@ -97,12 +102,9 @@ class EmulEnv:
             nt = len(tb)
         self._tb = tb
         self.N, self.stride = num_envs, legal_stride
-        slots = 16
-        if tb is not None:
-            slots = max(16, int(max((tb > 0).sum(1).max(), (tb < 0).sum(1).max())))
+        self.opponent, self.player_color, self.history_cap, self.moves_max = opponent, player_color, history_cap, moves_max
         self._h = lib().emul_env_create(num_envs, env_id_offset, seed, {"none": 0, "random": 1, "external": 2}[opponent],
-                                        int(player_color == "BLACK"), int(auto_reset), slots, history_cap, moves_max,
-                                        nt, _p(tb))
+                                        int(player_color == "BLACK"), int(auto_reset), 0, history_cap, moves_max, nt, _p(tb))
 
     def __del__(self):
         if getattr(self, "_h", None):
@@ -151,3 +153,34 @@ class EmulEnv:
         s = np.zeros(16, np.uint64)
         lib().emul_env_stats(self._h, _p(s))
         return s
+
+    def clone_from(self, source, index):
+        """env j becomes env index[j] of `source` for 0 <= index[j] < source.N; index < 0 leaves row j alone"""
+        mine, theirs = [(e.history_cap, e.opponent, e.player_color, e.moves_max, lib().emul_env_piece_slots(e._h))
+                        for e in (self, source)]
+        assert mine == theirs, "configuration mismatch: %r here, %r in the source" % (mine, theirs)
+        idx = np.ascontiguousarray(np.asarray(index, np.int32).reshape(self.N))
+        lib().emul_env_clone(self._h, source._h, idx.ctypes.data)
+
+    def sample_policy(self, logits, temperature=1.0, u32=None):
+        """logits: float32 [N, >= 4101], or uint16 [N, >= 4101] holding bf16 bit patterns (numpy rows may be padded: the row
+        stride is taken from the array).  -> (actions int32[N], logp float32[N])"""
+        assert logits.ndim == 2 and logits.shape[0] == self.N and logits.shape[1] >= 4101 and logits.strides[1] == logits.itemsize
+        dtype = {np.dtype(np.float32): 0, np.dtype(np.uint16): 1}[logits.dtype]
+        words = None if u32 is None else np.ascontiguousarray(np.asarray(u32).astype(np.uint32).reshape(self.N))
+        act, logp = np.zeros(self.N, np.int32), np.zeros(self.N, np.float32)
+        lib().emul_env_sample_policy(self._h, logits.ctypes.data, dtype, logits.strides[0] // logits.itemsize, float(temperature),
+                                     None if words is None else words.ctypes.data, act.ctypes.data, logp.ctypes.data)
+        return act, logp
+
+    def encode(self, dtype=np.uint8):
+        """-> (planes [N, 19, 64] of dtype float32, uint16 (bf16 bit patterns) or uint8, rep uint8 [N])"""
+        planes = np.full((self.N, 19, 64), 7, dtype)  # (a value no plane holds: every element must be written)
+        rep = np.full(self.N, 0xEE, np.uint8)
+        lib().emul_env_encode(self._h, planes.ctypes.data, _ENCODE_DTYPES[np.dtype(dtype)], rep.ctypes.data)
+        return planes, rep
+
+    def repetition_count(self):
+        rep = np.full(self.N, 0xEE, np.uint8)
+        lib().emul_env_encode(self._h, None, 0, rep.ctypes.data)
+        return rep

@@ -1,6 +1,6 @@
 // host_emul.cpp -- TEST INFRASTRUCTURE.  Compiles the device rules (gym_chess_b200/csrc/chess_core.cuh,
-// env_core.cuh) with g++ so that `pytest -m "not gpu"` can check the bitboard / step LOGIC against the oracle
-// on a box without a GPU.  It is never loaded by the product package; the product has no CPU path.
+// env_core.cuh) with g++ so that `pytest -m "not gpu"` can check the bitboard / step / clone / policy / encode LOGIC
+// against the oracle on a box without a GPU.  It is never loaded by the product package; the product has no CPU path.
 #include <stdint.h>
 #include <stdlib.h>
 #include <string.h>
@@ -150,11 +150,10 @@ void emul_env_destroy(EmulEnv* E) {
     free(E);
 }
 
+// slots 0 = automatic, as gcb_env_config.piece_slots
 EmulEnv* emul_env_create(int N, uint32_t env_offset, uint64_t seed, int opponent, int agent_black, int auto_reset, int slots,
                          int hist_cap, int moves_max, int n_templates, const int8_t* template_boards) {
-    static const int8_t def[64] = {-3, -5, -4, -2, -1, -4, -5, -3, -6, -6, -6, -6, -6, -6, -6, -6, 0, 0, 0, 0, 0, 0,
-                                   0,  0,  0,  0,  0,  0,  0,  0,  0,  0,  0,  0,  0,  0,  0,  0,  0, 0, 0, 0, 0, 0,
-                                   0,  0,  0,  0,  6,  6,  6,  6,  6,  6,  6,  6,  3,  5,  4,  2,  1, 4, 5, 3};
+    if (slots == 0) slots = auto_piece_slots(n_templates, template_boards);
     EmulEnv* E = (EmulEnv*)calloc(1, sizeof(EmulEnv));
     int T = n_templates > 0 ? n_templates : 1;
     EnvView& v = E->v;
@@ -172,7 +171,7 @@ EmulEnv* emul_env_create(int N, uint32_t env_offset, uint64_t seed, int opponent
     v.moves_max = moves_max, v.opponent = opponent, v.agent_black = agent_black, v.auto_reset = auto_reset;
     v.pps = 1 + (opponent == 1);
     for (int i = 0; i < T; i++)
-        make_template_one(i, n_templates > 0 ? template_boards : def, E->t_bb01, E->t_bb23, E->t_meta, E->t_zkey, E->t_tgt, E->t_cnt, slots);
+        make_template_one(i, n_templates > 0 ? template_boards : kDefaultBoard, E->t_bb01, E->t_bb23, E->t_meta, E->t_zkey, E->t_tgt, E->t_cnt, slots);
     StepIO io;
     memset(&io, 0, sizeof(io));
     io.tick = E->tick++, io.e_begin = 0, io.e_end = N, io.nsteps = 1;
@@ -234,6 +233,40 @@ void emul_env_export(EmulEnv* E, int8_t* boards, int32_t* info, uint16_t* legal,
 }
 
 void emul_env_stats(EmulEnv* E, uint64_t* out16) { memcpy(out16, E->v.stats, ST_COUNT * 8); }
+
+int emul_env_piece_slots(const EmulEnv* E) { return E->v.slots; }
+
+// the per-env clone (gcb_env_clone): the GCB_HD code of env_core.cuh that k_env_clone splits among the lanes of a warp, run
+// row by row.  index int32[dst N]: env d of dst becomes env index[d] of src for 0 <= index[d] < src N; other rows are left untouched
+void emul_env_clone(EmulEnv* dst, const EmulEnv* src, const int32_t* index) {
+    for (int d = 0; d < dst->v.N; d++) {
+        const int i = index[d];
+        if (i < 0 || i >= src->v.N) continue;
+        env_clone_one(dst->v, d, src->v, i);
+    }
+}
+
+// policy sampling (gcb_env_sample_policy): env_policy_sample_one, the serial form of the rule that k_env_policy_sample runs
+// with one warp per env.
+// logits [N][row_stride] of dtype 0 (fp32) / 1 (bf16 as uint16); words uint32[N] or NULL (Philox); logp may be NULL
+void emul_env_sample_policy(const EmulEnv* E, const void* logits, int dtype, long long row_stride, float temperature,
+                            const uint32_t* words, int32_t* actions, float* logp) {
+    for (int e = 0; e < E->v.N; e++) {
+        if (dtype == 1) env_policy_sample_one<1>(E->v, e, logits, row_stride, temperature, words, actions, logp);
+        else env_policy_sample_one<0>(E->v, e, logits, row_stride, temperature, words, actions, logp);
+    }
+}
+
+// the network-input encoder (gcb_env_encode): env_encode_one, the serial form of the rule that k_env_encode writes with one
+// warp per 32 envs.
+// planes [N][19][64] of dtype 0 (fp32) / 1 (bf16 as uint16) / 2 (uint8), or NULL; rep uint8[N] or NULL
+void emul_env_encode(const EmulEnv* E, void* planes, int dtype, uint8_t* rep) {
+    for (int e = 0; e < E->v.N; e++) {
+        if (dtype == 1) env_encode_one<1>(E->v, e, static_cast<uint16_t*>(planes), rep);
+        else if (dtype == 2) env_encode_one<2>(E->v, e, static_cast<uint8_t*>(planes), rep);
+        else env_encode_one<0>(E->v, e, static_cast<float*>(planes), rep);
+    }
+}
 
 // the 16-bit result record of the packed step forms (gcb_env_step_packed)
 uint16_t emul_pack_result(int reward, int done, uint32_t flags) { return pack_result(reward, done != 0, flags); }

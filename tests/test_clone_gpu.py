@@ -1,18 +1,13 @@
 """Per-env clone on the GPU (gcb_env_clone / BatchedChessEnv.clone_from, kernel k_env_clone): against the oracle, at full
 size against the source envs themselves, in-object, with a registered mask output, argument checks, and the memory-safety
 net (guard regions, CHECKED build) in a subprocess."""
-import json
-import os
-import subprocess
-import sys
-
 import numpy as np
 import pytest
 
 from tests import clone_helpers as ch
+from tests import memsafety_exercise as mx
 
 pytestmark = pytest.mark.gpu
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 CHK_CLONE_INDEX, CHK_CLONE_ALIAS = 6, 7
 
 
@@ -197,34 +192,22 @@ def test_configuration_mismatch_raises_value_error():
         D.clone_from(S, np.arange(16).reshape(2, 8))
 
 
-def _memsafety(mode, variant=None):
-    from gym_chess_b200 import _lib
-
-    env = dict(os.environ)
-    if variant:
-        env["GYMCHESS_B200_LIB"] = _lib.build(variant=variant)
-    out = subprocess.run([sys.executable, os.path.join(ROOT, "tests", "clone_memsafety.py"), mode], env=env,
-                         capture_output=True, text=True, timeout=900)
-    assert out.returncode == 0, out.stderr[-2000:]
-    return json.loads(out.stdout.strip().splitlines()[-1])
-
-
 def test_clone_guard_regions_stay_intact():
-    res = _memsafety("valid")
+    res = mx.run()["clone_valid"]
     assert res["guard_bad_bytes"] == 0 and res["violations"] == 0, res
 
 
 def test_checked_build_reports_no_violation_for_valid_clones():
-    res = _memsafety("valid", "checked")
+    res = mx.run("checked")["clone_valid"]
     assert res["checked"] == 1 and res["violations"] == 0 and res["guard_bad_bytes"] == 0, res
 
 
 def test_checked_build_flags_an_out_of_range_index_and_leaves_the_row():
-    res = _memsafety("out_of_range", "checked")
+    res = mx.run("checked")["clone_out_of_range"]
     assert res["checked"] == 1 and res["violations"] == 1 << CHK_CLONE_INDEX and res["untouched"], res
     assert res["guard_bad_bytes"] == 0
 
 
 def test_checked_build_flags_aliasing():
-    res = _memsafety("alias", "checked")
+    res = mx.run("checked")["clone_alias"]
     assert res["checked"] == 1 and res["violations"] == 1 << CHK_CLONE_ALIAS and res["guard_bad_bytes"] == 0, res

@@ -1,5 +1,5 @@
 """Per-env clone (gcb_env_clone / BatchedChessEnv.clone_from) on the host emulation: the GCB_HD code of env_core.cuh that
-k_env_clone runs, compiled with g++ (tests/host_emul/clone_emul.cpp) and checked against the oracle and against the
+k_env_clone runs, compiled with g++ (tests/host_emul/host_emul.cpp) and checked against the oracle and against the
 source envs themselves.  The same checks on the GPU are in test_clone_gpu.py."""
 import numpy as np
 import pytest
@@ -7,7 +7,7 @@ import pytest
 from oracle import oracle as orc
 from tests import clone_helpers as ch
 from tests import parity_helpers as ph
-from tests.host_emul import clone_emul as ce
+from tests.host_emul import emul
 
 F_REPETITION = 4
 
@@ -18,7 +18,7 @@ SHUFFLE = [NF3, NF6, NG1, NG8] * 2 + [NF3]
 
 @pytest.mark.parametrize("opponent,color", [("none", "WHITE"), ("random", "WHITE"), ("random", "BLACK")])
 def test_clone_vs_oracle(opponent, color):
-    ch.check_clone_vs_oracle(ce.EmulEnv, opponent, color, 192, np.random.RandomState(5))
+    ch.check_clone_vs_oracle(emul.EmulEnv, opponent, color, 192, np.random.RandomState(5))
 
 
 def test_clone_external_opponent_continues_like_its_source():
@@ -26,9 +26,9 @@ def test_clone_external_opponent_continues_like_its_source():
     continue exactly like their sources"""
     rng = np.random.RandomState(6)
     kw = dict(opponent="external", player_color="BLACK", auto_reset=False)
-    S = ce.EmulEnv(96, seed=1, **kw)
+    S = emul.EmulEnv(96, seed=1, **kw)
     ch.drive_pair(S, S, np.full(96, -1, np.int32), 30, rng, external=True)  # (plays the source only)
-    D = ce.EmulEnv(96, seed=2, env_id_offset=500, **kw)
+    D = emul.EmulEnv(96, seed=2, env_id_offset=500, **kw)
     S.step_index(rng.randint(0, 2 ** 32, size=96, dtype=np.uint64).astype(np.uint32))   # now a bot ply is owed
     assert (S.export()[1][:, 14] == 1).any()
     idx = rng.permutation(96).astype(np.int32)
@@ -50,14 +50,14 @@ def test_repetition_window_is_carried_across_the_clone():
     """5 plies of the knight shuffle, clone, 4 more plies on the clone: the 3-fold repetition fires at ply 9 as it does on
     the source.  A state import of the same board starts a new episode with an empty window and does NOT fire: this is
     why the clone exists."""
-    S = _shuffle_env(ce.EmulEnv, seed=1)
+    S = _shuffle_env(emul.EmulEnv, seed=1)
     for a in SHUFFLE[:5]:
         r, d, f = S.step(np.array([a], np.int32))[:3]
         assert not d[0] and not f[0] & F_REPETITION
-    D = _shuffle_env(ce.EmulEnv, seed=77, env_id_offset=9)
+    D = _shuffle_env(emul.EmulEnv, seed=77, env_id_offset=9)
     D.clone_from(S, np.array([0], np.int32))
     boards, info, _ = S.export()
-    I = _shuffle_env(ce.EmulEnv, seed=1)
+    I = _shuffle_env(emul.EmulEnv, seed=1)
     I.set_state(boards, info[:, 0].astype(np.int8), info[:, 1:5].astype(np.uint8), info[:, 8].astype(np.int32))
     for k, a in enumerate(SHUFFLE[5:]):
         last = k == len(SHUFFLE) - 6
@@ -78,7 +78,7 @@ def test_clone_continues_exactly_like_its_source(boards, history_cap, moves_max,
     N = 128
     kw = dict(opponent="none", auto_reset=False, history_cap=history_cap, moves_max=moves_max,
               initial_boards=ph.endgame_boards() if boards == "endgames" else None)
-    S = ce.EmulEnv(N, seed=3, **kw)
+    S = emul.EmulEnv(N, seed=3, **kw)
     # long windows: up to 180 steps before the clone, rows staggered by resets
     for rnd in range(3):
         for _ in range(60):
@@ -89,7 +89,7 @@ def test_clone_continues_exactly_like_its_source(boards, history_cap, moves_max,
         idx = np.full(N, -1, np.int32)
         idx[N // 2:] = np.arange(N // 2)
     else:
-        D = ce.EmulEnv(N, seed=4, env_id_offset=7000, **kw)
+        D = emul.EmulEnv(N, seed=4, env_id_offset=7000, **kw)
         idx = rng.permutation(N).astype(np.int32)
     assert S.export()[1][:, 12].max() > (8 if history_cap == 8 else 20)  # non-trivial windows are being cloned
     st_s, st_d = S.stats(), D.stats()
@@ -104,8 +104,8 @@ def test_clone_continues_exactly_like_its_source(boards, history_cap, moves_max,
 
 def test_clone_leaves_unselected_and_out_of_range_rows_alone():
     rng = np.random.RandomState(9)
-    S = ce.EmulEnv(40, opponent="none", seed=3)
-    D = ce.EmulEnv(50, opponent="none", seed=4)
+    S = emul.EmulEnv(40, opponent="none", seed=3)
+    D = emul.EmulEnv(50, opponent="none", seed=4)
     for _ in range(20):
         S.step_sampled()
         D.step_sampled()

@@ -9,36 +9,6 @@ from tests import parity_helpers as ph
 from tests.host_emul import emul
 
 
-class EmulAdapter:
-    def __init__(self, N, **kw):
-        self.N = N
-        self.e = emul.EmulEnv(N, **kw)
-
-    def step(self, a):
-        return self.e.step(a)
-
-    def step_index(self, u):
-        return self.e.step_index(u)
-
-    def step_sampled(self):
-        return self.e.step_sampled()
-
-    def bot_ply(self, a):
-        return self.e.bot_ply(a)
-
-    def export(self):
-        return self.e.export()
-
-    def reset(self, mask=None):
-        return self.e.reset(mask)
-
-    def set_state(self, *a):
-        return self.e.set_state(*a)
-
-    def stats(self):
-        return self.e.stats()
-
-
 def _mg(boards, players, rights, attack):
     return emul.movegen(boards, players, rights, attack)
 
@@ -88,13 +58,13 @@ def test_philox_matches_oracle():
 
 @pytest.mark.parametrize("opponent,color", [("none", "WHITE"), ("random", "WHITE"), ("random", "BLACK")])
 def test_env_sampled_vs_oracle(opponent, color):
-    env = EmulAdapter(12, opponent=opponent, player_color=color, seed=21, auto_reset=True)
+    env = emul.EmulEnv(12, opponent=opponent, player_color=color, seed=21, auto_reset=True)
     st = ph.check_sampled_vs_oracle(env, opponent, color, 21, 650)
     assert st[2] > 0  # episodes ended (cap / mate / repetition / wedge all occur in 650 steps x 12 envs)
 
 
 def test_env_index_mode_and_offset_vs_oracle():
-    env = EmulAdapter(8, opponent="none", seed=5, auto_reset=True, env_id_offset=1000)
+    env = emul.EmulEnv(8, opponent="none", seed=5, auto_reset=True, env_id_offset=1000)
     ph.check_sampled_vs_oracle(env, "none", "WHITE", 5, 200, env_id_offset=1000, mode="index", rng=np.random.RandomState(1))
 
 
@@ -106,7 +76,7 @@ def test_env_edge_templates_vs_oracle(golden):
     boards = np.array(boards, np.int8)
     assert len(boards) >= 15
     for opponent, color in (("none", "WHITE"), ("random", "WHITE"), ("random", "BLACK")):
-        env = EmulAdapter(len(boards) * 2, opponent=opponent, player_color=color, seed=8, auto_reset=True, initial_boards=boards)
+        env = emul.EmulEnv(len(boards) * 2, opponent=opponent, player_color=color, seed=8, auto_reset=True, initial_boards=boards)
         ph.check_sampled_vs_oracle(env, opponent, color, 8, 260, boards=boards)
 
 
@@ -115,12 +85,12 @@ def test_env_no_autoreset_wedge_and_done_behaviour():
     K, Q = 1, 2
     b = np.zeros((8, 8), np.int8)
     b[0, 0], b[3, 1], b[2, 2] = -K, Q, K
-    env = EmulAdapter(1, opponent="none", auto_reset=False, initial_boards=b)
+    env = emul.EmulEnv(1, opponent="none", auto_reset=False, initial_boards=b)
     r, d, f, _, _ = env.step([orc.str_to_action("b5b6")])
     assert (r[0], d[0], f[0] & 16) == (-10, 0, 16)
     r, d, f, _, _ = env.step([0])
     assert (r[0], d[0], f[0] & 1) == (-10, 0, 1)
-    env = EmulAdapter(1, opponent="none", auto_reset=False, initial_boards=b)
+    env = emul.EmulEnv(1, opponent="none", auto_reset=False, initial_boards=b)
     r, d, f, _, _ = env.step([orc.str_to_action("b5b7")])
     assert (r[0], d[0], f[0] & 2) == (90, 1, 2)
     r, d, f, _, _ = env.step([0])
@@ -132,7 +102,7 @@ def test_env_replays_real_chess_v2_selfplay_games(golden):
     for t in golden["trajectories"]:
         if t["opponent"] != "none":
             continue
-        n += ph.check_trajectory_replay(lambda ib: EmulAdapter(1, opponent="none", auto_reset=False, initial_boards=ib), t)
+        n += ph.check_trajectory_replay(lambda ib: emul.EmulEnv(1, opponent="none", auto_reset=False, initial_boards=ib), t)
     assert n > 5000
 
 
@@ -144,7 +114,7 @@ def test_external_opponent_replays_real_chess_v2_bot_games(golden):
         if t["opponent"] != "random":
             continue
         n += ph.check_external_bot_replay(
-            lambda ib, color: EmulAdapter(1, opponent="external", player_color=color, auto_reset=False, initial_boards=ib), t)
+            lambda ib, color: emul.EmulEnv(1, opponent="external", player_color=color, auto_reset=False, initial_boards=ib), t)
     assert n > 4000
 
 
@@ -158,7 +128,7 @@ def test_many_piece_templates_use_more_slots():
         boards[i, sq[22:40]] = -rng.choice([2, 3, 4, 5, 6], size=18)
         boards[i, sq[40]], boards[i, sq[41]] = 1, -1
     for opponent, color in (("none", "WHITE"), ("random", "BLACK")):
-        env = EmulAdapter(12, opponent=opponent, player_color=color, seed=11, auto_reset=True, initial_boards=boards)
+        env = emul.EmulEnv(12, opponent=opponent, player_color=color, seed=11, auto_reset=True, initial_boards=boards)
         ph.check_sampled_vs_oracle(env, opponent, color, 11, 150, boards=boards, compare_every=10)
 
 
@@ -168,7 +138,7 @@ def test_more_than_255_legal_moves():
     boards = ph.queen_heavy_boards()
     n_max = max(orc.OracleEnv(b, "WHITE", "none", 1, 0).view()["n_legal"] for b in boards)
     assert n_max > 255
-    env = EmulAdapter(8, opponent="none", seed=21, auto_reset=True, initial_boards=boards, legal_stride=512)
+    env = emul.EmulEnv(8, opponent="none", seed=21, auto_reset=True, initial_boards=boards, legal_stride=512)
     ph.check_sampled_vs_oracle(env, "none", "WHITE", 21, 60, boards=boards, compare_every=5)
 
 
@@ -176,11 +146,11 @@ def test_endgames_with_long_repetition_windows():
     """BASELINE.json configs[4]: repetition-heavy endgames, move cap lifted, 512-slot ring: the Bloom-gated ring scan
     must find every 3-fold the reference's dict finds (windows grow to hundreds of plies here)"""
     boards = ph.endgame_boards()
-    env = EmulAdapter(21, opponent="none", seed=17, auto_reset=True, initial_boards=boards, moves_max=250, history_cap=512)
+    env = emul.EmulEnv(21, opponent="none", seed=17, auto_reset=True, initial_boards=boards, moves_max=250, history_cap=512)
     st = ph.check_sampled_vs_oracle(env, "none", "WHITE", 17, 900, boards=boards, compare_every=50, moves_max=250)
     assert st[4] > 20 and st[11] == 0  # repetitions happened, no ring overflow
     assert st[14] / st[1] > 20         # mean window far above random play's ~6
-    env = EmulAdapter(14, opponent="random", player_color="BLACK", seed=18, auto_reset=True, initial_boards=boards, history_cap=512)
+    env = emul.EmulEnv(14, opponent="random", player_color="BLACK", seed=18, auto_reset=True, initial_boards=boards, history_cap=512)
     ph.check_sampled_vs_oracle(env, "random", "BLACK", 18, 500, boards=boards, compare_every=50)  # BLACK agent: no cap (Q12)
 
 
@@ -190,14 +160,14 @@ def test_move_sets_of_the_reference_pure_python_env(golden):
 
 @pytest.mark.parametrize("opponent,color", [("none", "WHITE"), ("random", "WHITE"), ("random", "BLACK")])
 def test_state_import_vs_oracle(opponent, color):
-    env = EmulAdapter(16, opponent=opponent, player_color=color, seed=41, auto_reset=True)
+    env = emul.EmulEnv(16, opponent=opponent, player_color=color, seed=41, auto_reset=True)
     ph.check_state_import_vs_oracle(env, opponent, color, 41, np.random.RandomState(6))
 
 
 @pytest.mark.parametrize("opponent,color,auto_reset", [("none", "WHITE", True), ("random", "WHITE", True), ("random", "BLACK", True),
                                                          ("none", "WHITE", False), ("random", "WHITE", False)])
 def test_external_actions_incl_invalid_vs_oracle(opponent, color, auto_reset):
-    env = EmulAdapter(10, opponent=opponent, player_color=color, seed=77, auto_reset=auto_reset)
+    env = emul.EmulEnv(10, opponent=opponent, player_color=color, seed=77, auto_reset=auto_reset)
     st = ph.check_external_actions_vs_oracle(env, opponent, color, 77, 420, np.random.RandomState(8), auto_reset)
     assert st[7] > 0  # invalid actions occurred
 

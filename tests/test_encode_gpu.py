@@ -4,23 +4,19 @@ external opponent), against the NumPy reference of tests/encode_helpers.py at 30
 invariant (plane 18 <=> the next ply reports F_REPETITION) over 524,288 envs, the pure-read guarantee, out= into a slice of a
 rollout buffer, clones, argument errors and the memory-safety net (guard regions, CHECKED build) in a subprocess."""
 import ctypes as C
-import json
-import os
-import subprocess
-import sys
 
 import numpy as np
 import pytest
 
 from tests import encode_helpers as eh
 from tests import external_helpers as xh
+from tests import memsafety_exercise as mx
 from tests import parity_helpers as ph
-from tests.host_emul import encode_emul as ee
+from tests.host_emul import emul
 from tests.test_clone_gpu import GpuEnv
 from tests.test_external_opponent_gpu import GpuExternal
 
 pytestmark = pytest.mark.gpu
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 N_BIG = 100_003
 F_REPETITION, F_CAP = 4, 8
 GCB_E_ARG = -2
@@ -51,7 +47,7 @@ class _Pair:
         from gym_chess_b200 import BatchedChessEnv
 
         self.g = BatchedChessEnv(N, legal_stride=256, **kw)
-        self.h = ee.EmulEnv(N, legal_stride=256, **kw)
+        self.h = emul.EmulEnv(N, legal_stride=256, **kw)
         self.N = N
 
     def compare(self, tag):
@@ -262,23 +258,11 @@ def test_argument_errors():
     assert torch.equal(good, env.encode()) and torch.equal(rep, env.repetition_count())
 
 
-def _memsafety(variant=None):
-    from gym_chess_b200 import _lib
-
-    env = dict(os.environ)
-    if variant:
-        env["GYMCHESS_B200_LIB"] = _lib.build(variant=variant)
-    out = subprocess.run([sys.executable, os.path.join(ROOT, "tests", "encode_memsafety.py")], env=env,
-                         capture_output=True, text=True, timeout=900)
-    assert out.returncode == 0, out.stderr[-2000:]
-    return json.loads(out.stdout.strip().splitlines()[-1])
-
-
 def test_encode_guard_regions_stay_intact():
-    res = _memsafety()
+    res = mx.run()["encode"]
     assert res["guard_bad_bytes"] == 0 and res["out_guard_bad"] == 0 and res["violations"] == 0, res
 
 
 def test_checked_build_reports_no_violation_for_encodes():
-    res = _memsafety("checked")
+    res = mx.run("checked")["encode"]
     assert res["checked"] == 1 and res["violations"] == 0 and res["guard_bad_bytes"] == 0 and res["out_guard_bad"] == 0, res

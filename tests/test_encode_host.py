@@ -1,5 +1,5 @@
 """Network-input encoder (gcb_env_encode / BatchedChessEnv.encode) on the host emulation: env_encode_one of env_core.cuh
-compiled with g++ (tests/host_emul/encode_emul.cpp), compared byte for byte with the NumPy reference of
+compiled with g++ (tests/host_emul/host_emul.cpp), compared byte for byte with the NumPy reference of
 tests/encode_helpers.py (planes from the oracle's view, the repetition count from the oracle's saved_boards history) in
 self-play from the default board (with takebacks) and sampled from the endgame templates, against the random bot with either
 colour, with an external opponent while a bot ply is owed, after state imports, for clones and for done envs without
@@ -11,7 +11,7 @@ from oracle import oracle as orc
 from tests import encode_helpers as eh
 from tests import external_helpers as xh
 from tests import parity_helpers as ph
-from tests.host_emul import encode_emul as ee
+from tests.host_emul import emul
 from tests.test_external_opponent_host import EmulExternal
 
 F_REPETITION = 4
@@ -68,7 +68,7 @@ def _run_takebacks(E, O, rng, tag):
 def test_encode_matches_reference_in_self_play_and_against_the_bot(opponent, color, boards, driver, steps, min_counts):
     N, seed = 128, 13
     tb = ph.endgame_boards() if boards == "endgames" else None
-    E = ee.EmulEnv(N, opponent=opponent, player_color=color, seed=seed, initial_boards=tb)
+    E = emul.EmulEnv(N, opponent=opponent, player_color=color, seed=seed, initial_boards=tb)
     O = _oracles(N, tb, color, opponent, seed)
     for o in O:
         o.last_move = [None, None]
@@ -85,20 +85,12 @@ def test_encode_matches_reference_in_self_play_and_against_the_bot(opponent, col
     assert seen[1] >= min_counts[0] and seen[2] >= min_counts[1], seen
 
 
-class EncodeExternal(EmulExternal):
-    """the external-opponent adapter of test_external_opponent_host.py on an emulation env that also encodes"""
-
-    def __init__(self, N, **kw):
-        self.N = N
-        self.e = ee.EmulEnv(N, opponent="external", legal_stride=256, **kw)
-
-
 @pytest.mark.parametrize("color", ["WHITE", "BLACK"])
 def test_encode_external_opponent_while_a_bot_ply_is_owed(color):
     """the env encodes the side to move: the bot while a ply is owed (after the agent's ply), the agent otherwise"""
     N, seed = 128, 5
     tb = ph.endgame_boards()
-    env = EncodeExternal(N, player_color=color, seed=seed, auto_reset=True, moves_max=149, initial_boards=tb)
+    env = EmulExternal(N, player_color=color, seed=seed, auto_reset=True, moves_max=149, initial_boards=tb)
     models = xh.make_models(N, color, seed, True, 149, tb)
     rng = np.random.RandomState(17 + len(color))
     seen, owed_rows = np.zeros(3, np.int64), 0
@@ -117,7 +109,7 @@ def test_encode_external_opponent_while_a_bot_ply_is_owed(color):
 def test_encode_after_state_import_starts_with_count_zero():
     N, seed = 64, 7
     rng = np.random.RandomState(3)
-    E = ee.EmulEnv(N, opponent="none", seed=seed)
+    E = emul.EmulEnv(N, opponent="none", seed=seed)
     O = _oracles(N, None, "WHITE", "none", seed)
     tot = dict(steps=0, reward_sum=0, episodes=0)
     ph._run_sampled(E, O, seed, 60, tot)
@@ -144,7 +136,7 @@ def test_encode_done_envs_without_auto_reset():
     """auto_reset off: an env that ended (mate, repetition, wedged) keeps its last position and is encoded as it stands"""
     N, seed = 96, 19
     tb = ph.endgame_boards()
-    E = ee.EmulEnv(N, opponent="none", seed=seed, initial_boards=tb, auto_reset=False)
+    E = emul.EmulEnv(N, opponent="none", seed=seed, initial_boards=tb, auto_reset=False)
     O = _oracles(N, tb, "WHITE", "none", seed)
     tot, done_rows = dict(steps=0, reward_sum=0, episodes=0), 0
     for t in range(150):
@@ -158,14 +150,14 @@ def test_clone_encodes_like_its_source():
     rng = np.random.RandomState(21)
     N = 128
     kw = dict(opponent="none", auto_reset=False, history_cap=64, moves_max=250, initial_boards=ph.endgame_boards())
-    S = ee.EmulEnv(N, seed=3, **kw)
+    S = emul.EmulEnv(N, seed=3, **kw)
     for rnd in range(3):
         for _ in range(40):
             S.step_index(rng.randint(0, 2 ** 32, size=N, dtype=np.uint64).astype(np.uint32))
         S.reset((rng.rand(N) < 0.2).astype(np.uint8))
     for _ in range(25):
         S.step_index(rng.randint(0, 2 ** 32, size=N, dtype=np.uint64).astype(np.uint32))
-    D = ee.EmulEnv(N, seed=4, env_id_offset=7000, **kw)
+    D = emul.EmulEnv(N, seed=4, env_id_offset=7000, **kw)
     idx = rng.randint(0, N, size=N).astype(np.int32)
     idx[::5] = -1
     before = D.encode(np.uint8)
@@ -181,7 +173,7 @@ def test_clone_encodes_like_its_source():
 
 
 def test_knight_shuffle_sets_plane_17_after_4_plies_and_plane_18_after_8():
-    E = ee.EmulEnv(1, opponent="none", auto_reset=False, seed=1)
+    E = emul.EmulEnv(1, opponent="none", auto_reset=False, seed=1)
     expected = [0, 0, 0, 0, 1, 1, 1, 1, 2]  # the count of the board each ply is played FROM
     for k, a in enumerate(SHUFFLE):
         planes, rep = E.encode(np.uint8)
@@ -192,7 +184,7 @@ def test_knight_shuffle_sets_plane_17_after_4_plies_and_plane_18_after_8():
 
 
 def test_encode_is_a_pure_read():
-    E = ee.EmulEnv(64, opponent="random", seed=12, initial_boards=ph.endgame_boards())
+    E = emul.EmulEnv(64, opponent="random", seed=12, initial_boards=ph.endgame_boards())
     for _ in range(30):
         E.step_sampled()
     before = E.export(), E.stats()

@@ -8,43 +8,24 @@
     read-modify-write of warps that lie wholly past the env range (value-preserving, so guard bytes cannot see it) -- and
     the checks MUST flag it: the net catches that class of bug.
 """
-import json
-import os
-import subprocess
-import sys
-
 import pytest
 
+from tests import memsafety_exercise as mx
+
 pytestmark = pytest.mark.gpu
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-SIZES = [1, 33, 64, 160, 3000, 70001, 131149]
 
 
 def test_guard_regions_stay_intact_on_the_product_build():
-    from tests import memsafety_exercise as mx
-
-    res = mx.exercise(SIZES)
-    os.environ.pop("GCB_GUARD_BYTES", None)
+    res = mx.run()["steps"]
     assert res["checked"] == 0 and res["guard_bad_bytes"] == 0 and res["violations"] == 0, res
 
 
-def _run_variant(variant, sizes, quick=False):
-    from gym_chess_b200 import _lib
-
-    so = _lib.build(variant=variant)
-    env = dict(os.environ, GYMCHESS_B200_LIB=so)
-    cmd = [sys.executable, os.path.join(ROOT, "tests", "memsafety_exercise.py"), ",".join(map(str, sizes))] + (["quick"] if quick else [])
-    out = subprocess.run(cmd, env=env, capture_output=True, text=True, timeout=900)
-    assert out.returncode == 0, out.stderr[-2000:]
-    return json.loads(out.stdout.strip().splitlines()[-1])
-
-
 def test_checked_build_reports_no_index_violation():
-    res = _run_variant("checked", SIZES)
+    res = mx.run("checked")["steps"]
     assert res["checked"] == 1 and res["violations"] == 0 and res["guard_bad_bytes"] == 0, res
 
 
 def test_checked_build_catches_the_reintroduced_stat_row_bug():
-    res = _run_variant("checked_selftest", [64, 160], quick=True)
+    res = mx.run("checked_selftest")["steps_quick"]
     assert res["checked"] == 1 and res["violations"] & 1, res          # bit 0 = CHK_STAT_ROW
     assert res["guard_bad_bytes"] == 0                                 # ... which guard bytes alone cannot see (it adds 0)

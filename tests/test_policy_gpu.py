@@ -4,18 +4,14 @@ either agent colour, external opponent for both the agent and the owed bot ply),
 step_policy against sample_policy + step, the sampled distribution at 1,048,576 draws, argument errors, a registered mask
 output, and the memory-safety net (guard regions, CHECKED build) in a subprocess."""
 import ctypes as C
-import json
-import os
-import subprocess
-import sys
 
 import numpy as np
 import pytest
 
+from tests import memsafety_exercise as mx
 from tests import policy_helpers as pp
 
 pytestmark = pytest.mark.gpu
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 N_BIG = 100_003
 F_BOT_PENDING = 64
 
@@ -226,23 +222,11 @@ def test_sample_is_a_pure_read_of_state_statistics_and_mask_output():
     assert all((p == q).all() for p, q in zip(before, env.export_numpy()))
 
 
-def _memsafety(variant=None):
-    from gym_chess_b200 import _lib
-
-    env = dict(os.environ)
-    if variant:
-        env["GYMCHESS_B200_LIB"] = _lib.build(variant=variant)
-    out = subprocess.run([sys.executable, os.path.join(ROOT, "tests", "policy_memsafety.py")], env=env,
-                         capture_output=True, text=True, timeout=900)
-    assert out.returncode == 0, out.stderr[-2000:]
-    return json.loads(out.stdout.strip().splitlines()[-1])
-
-
 def test_policy_guard_regions_stay_intact():
-    res = _memsafety()
+    res = mx.run()["policy"]
     assert res["guard_bad_bytes"] == 0 and res["out_guard_bad"] == 0 and res["violations"] == 0, res
 
 
 def test_checked_build_reports_no_violation_for_policy_samples():
-    res = _memsafety("checked")
+    res = mx.run("checked")["policy"]
     assert res["checked"] == 1 and res["violations"] == 0 and res["guard_bad_bytes"] == 0 and res["out_guard_bad"] == 0, res

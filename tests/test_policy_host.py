@@ -1,5 +1,5 @@
 """Policy sampling (gcb_env_sample_policy / BatchedChessEnv.sample_policy) on the host emulation: env_policy_sample_one of
-env_core.cuh compiled with g++ (tests/host_emul/policy_emul.cpp), checked against the float64 reference of
+env_core.cuh compiled with g++ (tests/host_emul/host_emul.cpp), checked against the float64 reference of
 tests/policy_helpers.py on oracle self-play, golden and crafted positions.  The same checks on the GPU are in
 test_policy_gpu.py."""
 import numpy as np
@@ -7,13 +7,13 @@ import pytest
 
 from tests import parity_helpers as ph
 from tests import policy_helpers as ph_pol
-from tests.host_emul import policy_emul as pe
+from tests.host_emul import emul
 
 RESIGN = 4100
 
 
 def _imported(boards, players, rights, seed=3, **kw):
-    E = pe.EmulEnv(len(boards), opponent="none", seed=seed, auto_reset=False, **kw)
+    E = emul.EmulEnv(len(boards), opponent="none", seed=seed, auto_reset=False, **kw)
     E.set_state(boards, players, rights)
     return E
 
@@ -28,7 +28,7 @@ def _golden_env():
 
 @pytest.mark.parametrize("opponent,color", [("none", "WHITE"), ("random", "WHITE"), ("random", "BLACK")])
 def test_policy_matches_reference_on_selfplay(opponent, color):
-    E = pe.EmulEnv(256, opponent=opponent, player_color=color, seed=11, env_id_offset=1000)
+    E = emul.EmulEnv(256, opponent=opponent, player_color=color, seed=11, env_id_offset=1000)
     rng = np.random.RandomState(2)
     for k in range(6):  # positions from several phases, both sides to move (the step count varies per env)
         for _ in range(int(rng.randint(3, 25))):
@@ -47,7 +47,7 @@ def test_policy_matches_reference_on_golden_positions():
 def test_policy_matches_reference_with_more_than_16_pieces():
     """crafted boards with 24 and 28 white pieces (more than 255 legal moves): slots beyond 16, many rounds of 32"""
     boards = ph.queen_heavy_boards()
-    E = pe.EmulEnv(8, opponent="none", seed=5, initial_boards=boards, auto_reset=False)
+    E = emul.EmulEnv(8, opponent="none", seed=5, initial_boards=boards, auto_reset=False)
     info = E.export()[1]
     assert (info[:, 9] > 255).all()
     ph_pol.check_env(E, 5, 0, np.random.RandomState(6))
@@ -168,7 +168,7 @@ def test_padded_row_stride():
 
 
 def test_sampling_is_a_pure_read():
-    E = pe.EmulEnv(64, opponent="random", seed=12)
+    E = emul.EmulEnv(64, opponent="random", seed=12)
     for _ in range(9):
         E.step_sampled()
     before = E.export(), E.stats()
