@@ -653,8 +653,9 @@ void gco_selfplay_mt(uint64_t seed, uint32_t env_lo, uint32_t env_hi, uint64_t n
     free(args);
 }
 
-/* ---- a persistent pool of self-play envs (bench.py --impl reference): burn-in once, then timed steps on the same
- * envs, so that the CPU arm measures the same steady-state mix of game phases as the GPU arm */
+/* ---- a persistent pool of envs: burn-in once, then timed steps on the same envs, so that the CPU arm of bench.py
+ * (--impl reference) measures the same steady-state mix of game phases as the GPU arm; configured like the CUDA env
+ * (opponent, agent colour, moves_max, template boards), it is also the reference of whole device batches */
 struct gco_pool {
     gco_env *envs;
     uint32_t n;
@@ -676,12 +677,40 @@ static void *pool_worker(void *p) {
     return NULL;
 }
 
-gco_pool *gco_pool_new(uint64_t seed, uint32_t env_lo, uint32_t env_hi) {
+gco_pool *gco_pool_new_cfg(uint64_t seed, uint32_t env_lo, uint32_t env_hi, int opponent, int agent_black, int moves_max,
+                           int n_templates, const int8_t *templates) {
     gco_pool *p = (gco_pool *)malloc(sizeof(gco_pool));
     p->n = env_hi - env_lo;
     p->envs = (gco_env *)malloc(sizeof(gco_env) * (size_t)p->n);
-    for (uint32_t i = 0; i < p->n; i++) gco_env_init(&p->envs[i], NULL, 0, GCO_OPP_NONE, seed, env_lo + i);
+    for (uint32_t i = 0; i < p->n; i++) {
+        const uint32_t id = env_lo + i; /* the device's template rule: global env id % n_templates */
+        const int8_t *board = (templates && n_templates > 0) ? templates + (size_t)(id % (uint32_t)n_templates) * 64 : NULL;
+        gco_env_init(&p->envs[i], board, agent_black, opponent, seed, id);
+        p->envs[i].moves_max = moves_max; /* (only steps read it: the reset inside gco_env_init does not) */
+    }
     return p;
+}
+
+gco_pool *gco_pool_new(uint64_t seed, uint32_t env_lo, uint32_t env_hi) {
+    return gco_pool_new_cfg(seed, env_lo, env_hi, GCO_OPP_NONE, 0, 149, 0, NULL);
+}
+
+/* ChessEnvV2.reset of the envs with mask[i] != 0, as the CUDA env's masked reset does it: a new episode (so a BLACK
+ * agent's opening ply is drawn with the new episode counter), the other envs keep their games */
+void gco_pool_reset(gco_pool *p, const uint8_t *mask) {
+    for (uint32_t i = 0; i < p->n; i++)
+        if (mask[i]) {
+            p->envs[i].episode++;
+            gco_env_reset(&p->envs[i]);
+        }
+}
+
+/* gco_env_view of every env: boards int8[n][64], info int32[n][16], legal uint16[n][stride] (the first min(n_legal,
+ * stride) entries of a row are written) */
+void gco_env_view(const gco_env *e, int8_t *board, int32_t *info, uint16_t *legal, int legal_cap);
+void gco_pool_export(const gco_pool *p, int8_t *boards, int32_t *info, uint16_t *legal, int stride) {
+    for (uint32_t i = 0; i < p->n; i++)
+        gco_env_view(&p->envs[i], boards + (size_t)i * 64, info + (size_t)i * 16, legal + (size_t)i * (size_t)stride, stride);
 }
 
 static void pool_run(gco_pool *p, uint64_t nsteps_per_env, uint32_t stagger, int threads, gco_stats *st);

@@ -264,22 +264,46 @@ def selfplay_mt(seed, env_lo, env_hi, nsteps_per_env, threads):
 
 
 class SelfplayPool:
-    """persistent self-play envs on the host threads (the CPU arm of bench.py)"""
+    """persistent envs with global ids [env_lo, env_hi) on the host threads: the CPU arm of bench.py (self-play from the
+    default board) and, configured like a BatchedChessEnv, the reference of a whole device batch.  Env id g starts from
+    initial_boards[g % T] (int8 [T,8,8] / [T,64], None: the default board)."""
 
-    def __init__(self, seed, env_lo, env_hi):
+    def __init__(self, seed, env_lo, env_hi, *, opponent="none", player_color=WHITE, moves_max=149, initial_boards=None):
         L = lib()
-        L.gco_pool_new.restype = C.c_void_p
-        L.gco_pool_new.argtypes = [C.c_uint64, C.c_uint32, C.c_uint32]
+        L.gco_pool_new_cfg.restype = C.c_void_p
+        L.gco_pool_new_cfg.argtypes = [C.c_uint64, C.c_uint32, C.c_uint32, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p]
         L.gco_pool_run.argtypes = [C.c_void_p, C.c_uint64, C.c_int, C.POINTER(Stats)]
         L.gco_pool_free.argtypes = [C.c_void_p]
         L.gco_pool_run_staggered.argtypes = [C.c_void_p, C.c_uint64, C.c_uint32, C.c_int, C.POINTER(Stats)]
-        self._h = L.gco_pool_new(seed, env_lo, env_hi)
+        L.gco_pool_reset.argtypes = [C.c_void_p, C.c_void_p]
+        L.gco_pool_export.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int]
+        self.n = int(env_hi) - int(env_lo)
+        tb, nt = None, 0
+        if initial_boards is not None:
+            tb = np.ascontiguousarray(np.asarray(initial_boards, dtype=np.int8).reshape(-1, 64))
+            nt = len(tb)
+        self._h = L.gco_pool_new_cfg(seed, env_lo, env_hi, {"none": 0, "random": 1}[opponent], int(player_color == BLACK),
+                                     int(moves_max), nt, None if tb is None else tb.ctypes.data)
 
     def run(self, nsteps_per_env, threads, stagger=0):
         """every env plays nsteps_per_env more steps (+ env index % stagger with stagger > 0: spreads the episode phases)"""
         st = Stats()
         lib().gco_pool_run_staggered(self._h, nsteps_per_env, stagger, threads, C.byref(st))
         return st.as_dict()
+
+    def reset(self, mask):
+        """ChessEnvV2.reset of the envs with mask[i] != 0 (a new episode each, like BatchedChessEnv.reset(mask))"""
+        m = np.ascontiguousarray(np.asarray(mask).reshape(self.n) != 0, dtype=np.uint8)
+        lib().gco_pool_reset(self._h, m.ctypes.data)
+
+    def export(self, stride=256):
+        """-> (boards int8 [n,64], info int32 [n,16], legal uint16 [n,stride]): OracleEnv.view() of every env, info in the
+        column order of OracleEnv.view(); the first min(n_legal, stride) entries of a legal row are the list, the rest 0"""
+        boards = np.zeros((self.n, 64), np.int8)
+        info = np.zeros((self.n, 16), np.int32)
+        legal = np.zeros((self.n, stride), np.uint16)
+        lib().gco_pool_export(self._h, boards.ctypes.data, info.ctypes.data, legal.ctypes.data, int(stride))
+        return boards, info, legal
 
     def __del__(self):
         if getattr(self, "_h", None):

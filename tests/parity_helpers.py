@@ -159,6 +159,25 @@ def _cmp_export(env, oracles, tag):
         assert mine == ref, "%s env %d: %s" % (tag, i, {k: (mine[k], ref[k]) for k in mine if mine[k] != ref[k]})
 
 
+def oracle_sampled_step(o, seed, env_id, tot, auto_reset=True, u=None):
+    """One sampled step of oracle env `o` (global id env_id): the device's Philox draw (or the caller's word u), the step,
+    and the device's auto-reset rule (a new episode when the step ended one or left no legal move).  Accumulates steps /
+    reward_sum / episodes in `tot`.  -> (action, reward, done, view after the step and before any reset, terminal)"""
+    v = o.view()
+    if u is None:
+        u = orc.draw_u32(seed, env_id, v["episode"], v["step_in_episode"], 0)
+    act = o.pick(u)
+    rr, dd, _ = o.step(act)
+    v2 = o.view()
+    terminal = dd or v2["n_legal"] == 0
+    tot["steps"] += 1
+    tot["reward_sum"] += rr
+    tot["episodes"] += int(terminal)
+    if terminal and auto_reset:
+        o.reset(v2["episode"] + 1)
+    return act, rr, dd, v2, terminal
+
+
 def _run_sampled(env, O, seed, steps, tot, auto_reset=True, env_id_offset=0, compare_every=25, mode="sampled", rng=None, tag=""):
     """`steps` steps on the device env and the SAME draws through the oracle envs O; compares every output of every
     step and the full state every `compare_every` steps; accumulates steps / reward_sum / episodes in `tot`."""
@@ -171,24 +190,59 @@ def _run_sampled(env, O, seed, steps, tot, auto_reset=True, env_id_offset=0, com
             words = rng.randint(0, 2 ** 32, size=N, dtype=np.uint64).astype(np.uint32)
             r, d, f, a, bot = env.step_index(words)
         for i, o in enumerate(O):
-            v = o.view()
-            u = orc.draw_u32(seed, env_id_offset + i, v["episode"], v["step_in_episode"], 0) if words is None else int(words[i])
-            act = o.pick(u)
-            rr, dd, raised = o.step(act)
-            v2 = o.view()
+            act, rr, dd, v2, terminal = oracle_sampled_step(o, seed, env_id_offset + i, tot, auto_reset,
+                                                            None if words is None else int(words[i]))
             assert (rr, dd) == (int(r[i]), bool(d[i])), "%sstep %d env %d: oracle %s device %s flags %d" % (tag, t, i, (rr, dd), (r[i], d[i]), f[i])
             if a is not None:
                 assert act == int(a[i]) and v2["last_bot_action"] == int(bot[i]), (tag, t, i, act, a[i], v2["last_bot_action"], bot[i])
-            terminal = dd or v2["n_legal"] == 0
             assert bool(f[i] & 32) == (terminal and auto_reset), (tag, t, i, int(f[i]), terminal)
             assert bool(f[i] & 16) == ((not dd) and v2["n_legal"] == 0), (tag, t, i, int(f[i]))
-            tot["steps"] += 1
-            tot["reward_sum"] += rr
-            tot["episodes"] += int(terminal)
-            if terminal and auto_reset:
-                o.reset(v2["episode"] + 1)
         if t % compare_every == 0 or t == steps - 1:
             _cmp_export(env, O, "%sstep %d" % (tag, t))
+
+
+# the info columns a device export (BatchedChessEnv.INFO_NAMES) and an oracle view (OracleEnv.view / SelfplayPool.export)
+# share, in this order; column 12 differs on purpose (the device's repetition window hist_len vs the oracle's hist_n)
+EXPORT_FIELDS = ("current_player", "wk", "wq", "bk", "bq", "wchk", "bchk", "done", "move_count", "n_legal", "episode",
+                 "step_in_episode")
+
+
+def oracle_views(O, stride=256):
+    """OracleEnv.view() of every env of O as the arrays of SelfplayPool.export(stride)"""
+    n = len(O)
+    boards, info, legal = np.zeros((n, 64), np.int8), np.zeros((n, 16), np.int32), np.zeros((n, stride), np.uint16)
+    for i, o in enumerate(O):
+        v = o.view()
+        boards[i] = v["board"]
+        info[i, : len(EXPORT_FIELDS)] = [v[k] for k in EXPORT_FIELDS]
+        k = min(v["n_legal"], stride)
+        legal[i, :k] = v["legal"][:k]
+    return boards, info, legal
+
+
+def check_export_arrays(got, ref, env_id_offset=0, tag="", show=8):
+    """got / ref: (boards [n,64], info [n,>=12], legal [n,stride]) with info columns EXPORT_FIELDS.  Board, every shared
+    info column and the legal list in order (its first min(n_legal, stride) entries) must agree for every env; on a
+    mismatch the message names the first `show` global env ids and, for each, the fields that differ."""
+    (b, info, legal), (rb, rinfo, rlegal) = got, ref
+    nf = len(EXPORT_FIELDS)
+    stride = min(legal.shape[1], rlegal.shape[1])
+    valid = np.arange(stride)[None, :] < np.minimum(rinfo[:, 9], stride)[:, None]
+    bad_board = (np.asarray(b) != rb).any(1)
+    bad_info = np.asarray(info)[:, :nf] != rinfo[:, :nf]
+    bad_legal = ((np.asarray(legal)[:, :stride] != rlegal[:, :stride]) & valid).any(1)
+    bad = bad_board | bad_info.any(1) | bad_legal
+    if not bad.any():
+        return
+    lines = []
+    for i in np.nonzero(bad)[0][:show]:
+        diff = {EXPORT_FIELDS[k]: (int(info[i, k]), int(rinfo[i, k])) for k in np.nonzero(bad_info[i])[0]}
+        if bad_board[i]:
+            diff["board"] = "squares %s" % np.nonzero(b[i] != rb[i])[0].tolist()
+        if bad_legal[i]:
+            diff["legal"] = "first difference at index %d" % int(np.argmax((legal[i, :stride] != rlegal[i, :stride]) & valid[i]))
+        lines.append("  env id %d (row %d): %s" % (env_id_offset + i, i, diff))
+    raise AssertionError("%s%d of %d envs differ (values: got, reference)\n%s" % (tag, int(bad.sum()), len(bad), "\n".join(lines)))
 
 
 def _check_totals(env, tot):

@@ -1,6 +1,7 @@
 """Pins the CPU oracle (oracle/gc_oracle.c) to the fixtures produced from the reference's REAL chess_v2.py and its own
 v2 test-suite (tests/golden/make_golden.py).  CPU only."""
 import numpy as np
+import pytest
 
 from oracle import oracle as orc
 from tests import parity_helpers as ph
@@ -157,3 +158,48 @@ def test_v1_castle_through_attack_vector():
         out, cnt = orc.movegen_batch(b[None], p, np.ones((1, 4), np.uint8), False)
         return [int(a) for a in out[0, : cnt[0]] if a >= 4096]
     ph.check_v1_castle_through_attack_vector(fn)
+
+
+POOL_CONFIGS = {  # opponent, player_color, moves_max, templates
+    "selfplay": ("none", orc.WHITE, 149, None),
+    "random-white": ("random", orc.WHITE, 149, None),
+    "random-black": ("random", orc.BLACK, 149, None),
+    "endgames": ("none", orc.WHITE, 250, "endgames"),
+}
+
+
+@pytest.mark.parametrize("config", list(POOL_CONFIGS))
+def test_pool_matches_the_per_env_driver(config):
+    """SelfplayPool (the host threads' reference of whole device batches) against OracleEnvs driven one sampled step at a
+    time by the driver of the device parity tests (parity_helpers.oracle_sampled_step): 64 envs with global ids from 1001,
+    self-play, the random bot for either agent colour and the endgame templates (env g starts from template g % 7), with a
+    masked reset in mid-game.  The exports and the pool's steps / reward_sum / episodes must be the driver's."""
+    opponent, color, moves_max, templates = POOL_CONFIGS[config]
+    boards = ph.endgame_boards() if templates else None
+    n, lo, seed = 64, 1001, 5
+    pool = orc.SelfplayPool(seed, lo, lo + n, opponent=opponent, player_color=color, moves_max=moves_max, initial_boards=boards)
+    O = [orc.OracleEnv(None if boards is None else boards[(lo + i) % len(boards)], color, opponent, seed, lo + i,
+                       moves_max=moves_max) for i in range(n)]
+    ph.check_export_arrays(pool.export(), ph.oracle_views(O), lo, "reset: ")
+    tot = dict(steps=0, reward_sum=0, episodes=0)
+    got = dict(steps=0, reward_sum=0, episodes=0)
+
+    def run(k, tag):
+        st = pool.run(k, 4)
+        for key in got:
+            got[key] += st[key]
+        for _ in range(k):
+            for i, o in enumerate(O):
+                ph.oracle_sampled_step(o, seed, lo + i, tot)
+        ph.check_export_arrays(pool.export(), ph.oracle_views(O), lo, tag)
+        assert got == tot, (tag, got, tot)
+
+    run(1, "1 step: ")
+    run(159, "160 steps: ")
+    mask = np.random.RandomState(3).rand(n) < 0.4
+    pool.reset(mask)
+    for i in np.nonzero(mask)[0]:
+        O[i].reset(O[i].view()["episode"] + 1)
+    ph.check_export_arrays(pool.export(), ph.oracle_views(O), lo, "masked reset: ")
+    run(160, "320 steps: ")
+    assert tot["episodes"] > 0
